@@ -17,6 +17,8 @@ begin + prefill + 255 fused decode steps + sampling = 32 x 9 x 256 tokens.
   vs_reference_gpu: the reference's fast GPU recipe (SDPA + static cache + CUDA-graph replay, INFERENCE.md:57-72) as a
                labelled PyTorch RESTATEMENT (oracle/decoder_static.py) timed on the same GPU in the same process
 `--impl reference` times the CPU port alone (the reference itself cannot be imported on the GPU box).
+`--dump-outputs DIR` writes what the last timed step computed (tokens, last logits, waveform) as .npy files; inputs, weights and
+sampling seeds depend only on the arguments, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 import argparse
@@ -112,6 +114,7 @@ class ClockSampler:
         if self.p is None:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         self.p.terminate()
+        self.p.wait()
         sm = sorted(int(float(r[0])) for r in self.rows if r and r[0].replace(".", "").isdigit())
         mx = [int(float(r[1])) for r in self.rows if len(r) > 1 and r[1].replace(".", "").isdigit()]
         names = ["hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown", "sw_power_cap"]
@@ -233,12 +236,9 @@ def run_reference(args, rank):
     if rank != 0:
         return
     vals = []
-    t0 = time.perf_counter()
     for i in range(args.warmup + args.steps):
-        if i >= 1 and time.perf_counter() - t0 > 150:   # keep the whole arm within a few minutes whatever K / W are
-            break
         m = cpu_port_measure(32, 1 if i < args.warmup else 3)
-        if i >= args.warmup or not vals:
+        if i >= args.warmup:
             vals.append(m)
     m = sorted(vals, key=lambda d: d["value"])[len(vals) // 2]
     v = m["value"]
@@ -346,6 +346,28 @@ def streaming_measure(model, dev, batch, steps, play_steps=20):
             "api": "model.generate(..., streamer=ParlerTTSStreamer(model, play_steps=20, incremental=True)) consumed on a thread"}
 
 
+DUMP_AUDIO_MAX = 8 << 20   # waveform samples written in full; above that a fixed sample, so a dump stays under 64 MB for every --config
+
+
+def dump_outputs(out_dir, shards, wav, suffix=""):
+    """What the last timed step computed, as float32 DIR/<name>.npy, so that two builds can be compared output for output:
+      tokens [B*K, L]: the token history of every (utterance, codebook) row, BOS column first (token ids are exact in float32)
+      logits [B*K, V]: the logits of the last decode step
+      audio  [B, samples]: the waveform of the generate() leg; when it holds more than DUMP_AUDIO_MAX samples, the samples at
+             DUMP_AUDIO_MAX sorted flat indices drawn with a fixed seed (the same indices for the same arguments)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"tokens": torch.cat([t for t, _ in shards]), "logits": torch.cat([lg for _, lg in shards])}
+    if wav is not None:
+        wav = wav.float()
+        if wav.numel() > DUMP_AUDIO_MAX:
+            idx = np.sort(np.random.default_rng(0).choice(wav.numel(), DUMP_AUDIO_MAX, replace=False))
+            wav = wav.flatten()[torch.from_numpy(idx)]
+        arrays["audio"] = wav
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), t.float().cpu().numpy())
+
+
 
 def main():
     ap = argparse.ArgumentParser()
@@ -358,7 +380,13 @@ def main():
     ap.add_argument("--no-gpu-reference", action="store_true")
     ap.add_argument("--no-dac", action="store_true")
     ap.add_argument("--decode-steps", type=int, default=None)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -416,7 +444,9 @@ def main():
             sess.decode_steps(n_dec - 1)
             if from_host:
                 outs.append(sess.raw_ids[:, :L].to("cpu", non_blocking=False))
-        return outs if from_host else None
+            elif args.dump_outputs:
+                outs.append((sess.raw_ids[:, :L].clone(), sess.logits.clone()))   # the next shard reuses the session's buffers
+        return outs
 
     def generate_pass(seed):
         """The public call: host tensors in, waveform on the host out (DAC decode inside generate())."""
@@ -452,13 +482,15 @@ def main():
     clocks = ClockSampler(local_rank)
     if rank == 0:
         clocks.start()
-    ms, launches, _ = timed(lambda s: one_pass(s, False))
-    clk = clocks.stop() if rank == 0 else None
+    try:
+        ms, launches, last_pass = timed(lambda s: one_pass(s, False))
+    finally:
+        clk = clocks.stop() if rank == 0 else None
     st = sess.state.cpu().tolist()
     assert st[0] == L, f"generation stopped early at length {st[0]} (expected {L})"
     fused = sess.fused
     ms_tok, _, _ = timed(lambda s: one_pass(s, True))
-    e2e_full = None
+    e2e_full, wav = None, None
     if not args.no_dac:
         if world > 1 and rank != 0:
             pass  # DAC weights arrived with the broadcast
@@ -466,6 +498,8 @@ def main():
         assert wav.shape == (B, (L - K) * 512), wav.shape
         e2e_full = (ms_e2e, wav.numel() * wav.element_size())
         sess = eng.session(Bs, P_LEN, S_LEN, P_LEN + L)  # (generate() may have re-created the session)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_pass, wav, f"_rank{rank}" if world > 1 else "")
 
     # decode-only timing for the roofline: the fused decode steps of one pass, T taken per step
     barrier()
