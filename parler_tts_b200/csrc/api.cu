@@ -39,7 +39,7 @@ struct ptts_session {
   const char* blob;
   char* ws;
   int sm_count;
-  bool pdl, use_graph;
+  bool use_graph;
   bool has_prompt_mask, has_enc_mask, begun, prefilled;
   ptts_gen_params gen;
   cudaStream_t cap_stream;
@@ -188,7 +188,6 @@ int ptts_session_create(const ptts_decoder_config* cfg, const void* blob, void* 
   cudaGetDevice(&dev);
   s->sm_count = 148;
   cudaDeviceGetAttribute(&s->sm_count, cudaDevAttrMultiProcessorCount, dev);
-  s->pdl = env_flag("PTTS_PDL", true);
   s->use_graph = env_flag("PTTS_GRAPH", true);
   s->graph_ready = false;
   s->exec = nullptr;
@@ -261,14 +260,13 @@ static bool setup_fused(ptts_session* s) {
   StepParams& p = s->sp;
   memset(&p, 0, sizeof(p));
   p.B = W.B; p.H = L.H; p.F = L.F; p.V = L.V; p.K = L.K; p.L = L.L; p.nh = L.nh; p.nkv = L.nkv; p.nckv = L.nckv;
-  p.S = W.S; p.P = W.P; p.Tmax = W.Tmax; p.rope = c.rope; p.act = c.activation; p.qkv_rows = L.qkv_rows; p.ckv_rows = L.ckv_rows;
+  p.S = W.S; p.P = W.P; p.Tmax = W.Tmax; p.rope = c.rope; p.act = c.activation; p.qkv_rows = L.qkv_rows;
   p.eps = c.layer_norm_eps; p.scale = 0.125f;
   p.blob = s->blob;
   p.embed = L.embed; p.pos = L.pos; p.layer0 = L.layer0; p.layer_stride = L.layer_stride;
-  p.ln1_w = L.ln1_w; p.ln1_b = L.ln1_b; p.wqkv = L.wqkv; p.wo = L.wo; p.ln2_w = L.ln2_w; p.ln2_b = L.ln2_b; p.wqc = L.wqc; p.woc = L.woc;
-  p.ln3_w = L.ln3_w; p.ln3_b = L.ln3_b; p.fc1 = L.fc1; p.fc2 = L.fc2;
+  p.wqkv = L.wqkv; p.wo = L.wo; p.wqc = L.wqc; p.woc = L.woc; p.fc1 = L.fc1; p.fc2 = L.fc2;
   p.c_qkv = L.c_qkv; p.c_qc = L.c_qc; p.c_fc1 = L.c_fc1; p.c_heads = L.c_heads;
-  p.final_ln_w = L.final_ln_w; p.final_ln_b = L.final_ln_b; p.heads = L.heads; p.rope_cos = L.rope_cos; p.rope_sin = L.rope_sin;
+  p.heads = L.heads; p.rope_cos = L.rope_cos; p.rope_sin = L.rope_sin;
   char* ws = s->ws;
   p.x = (bf16*)(ws + W.img_x); p.qkv = (bf16*)(ws + W.qkv); p.attn = (bf16*)(ws + W.img_attn); p.qc = (bf16*)(ws + W.qc); p.hbuf = (bf16*)(ws + W.img_h);
   p.logits = (float*)(ws + W.logits);
@@ -295,7 +293,6 @@ static bool setup_fused(ptts_session* s) {
   if ((int64_t)p.nt_h * L.F * 16 > wbytes) wbytes = (int64_t)p.nt_h * L.F * 16;
   if ((int64_t)p.nt_fc1 * L.H * 16 > wbytes) wbytes = (int64_t)p.nt_fc1 * L.H * 16;
   if ((int64_t)p.nt_heads * L.H * 16 > wbytes) wbytes = (int64_t)p.nt_heads * L.H * 16;
-  p.attn_floats_per_warp = 0;
   const int64_t att = (int64_t)8 * (2 * 2 * 32 * 64 * 2 + 3 * 64 * 4) + 4 * 128 * 4;  // 8 x attn_decode_smem_per_warp<bf16>() + pair exchange
   const int64_t budget = 215 * 1024 - 2816;  // step.cu ST_HEADER
   p.nbuf = (2 * tile + wbytes <= budget) ? 2 : 1;
@@ -310,7 +307,6 @@ static bool setup_fused(ptts_session* s) {
   if (p.sample_items > 9) return fused_declined(s, "vocab_size > 2304");
   p.do_sample_phase = 1;
   p.prof = s->prof;
-  { const char* d = getenv("PTTS_DBG"); p.dbg = d ? atoi(d) : 0; }
   // cluster variant (step2.cu) when the shape and the device allow it; PTTS_STEP=legacy keeps step.cu (A/B runs, cross-checks)
   for (int i = 0; i < 6; i++) { p.cp[i] = L.cp[i]; p.cp_slice[i] = L.cp_slice[i]; }
   p.cl_x = (bf16*)(ws + W.cl_x); p.cl_attn = (bf16*)(ws + W.cl_attn); p.cl_h = (bf16*)(ws + W.cl_h);
@@ -343,7 +339,7 @@ static int run_forward(ptts_session* s, cudaStream_t st, bool prefill, const voi
   const int B = W.B, P = W.P, S = W.S, H = L.H, D = PTTS_HEAD_DIM;
   const int q_len = prefill ? P + 1 : 1;
   const int M = B * q_len;
-  const bool pdl = s->pdl && !prefill;  // the one-off prefill stays on plain stream order
+  const bool pdl = !prefill;  // the one-off prefill stays on plain stream order
   const Ctrl* ctrl = prefill ? nullptr : (const Ctrl*)(s->ws + W.ctrl);
   const int es = L.es;
   char* ws = s->ws;
@@ -502,7 +498,7 @@ int ptts_decode_steps(ptts_session* s, int32_t n_steps, void* stream) {
     for (int i = 0; i < n_steps; i++) {
       if (int e = run_forward(s, st, false, nullptr, nullptr)) return e;
       s->launches++;
-      if (int e = launch_sample(sample_args(s), nullptr, st, s->pdl)) return e;
+      if (int e = launch_sample(sample_args(s), nullptr, st, true)) return e;
     }
     return PTTS_OK;
   }
@@ -511,7 +507,7 @@ int ptts_decode_steps(ptts_session* s, int32_t n_steps, void* stream) {
     const int64_t before = s->launches;
     PTTS_CHECK_CUDA(cudaStreamBeginCapture(s->cap_stream, cudaStreamCaptureModeThreadLocal));
     int e = run_forward(s, s->cap_stream, false, nullptr, nullptr);
-    if (!e) { s->launches++; e = launch_sample(sample_args(s), nullptr, s->cap_stream, s->pdl); }
+    if (!e) { s->launches++; e = launch_sample(sample_args(s), nullptr, s->cap_stream, true); }
     cudaGraph_t graph = nullptr;
     cudaError_t ce = cudaStreamEndCapture(s->cap_stream, &graph);
     s->launches = before;
@@ -713,7 +709,7 @@ int ptts_dac_decode(const ptts_dac_config* cfg, const void* blob, void* workspac
       }
     }
     const int cl = C >> cfg->n_blocks;
-    if (final_conv_supported(cl) && env_flag("PTTS_DAC_FINAL_FAST", true))   // one thread per output sample (dac.cu)
+    if (final_conv_supported(cl))   // one thread per output sample (dac.cu)
       return launch_final_conv_tanh(act, tpp(ti + 1), tpp(ti + 2), audio_out, cl, Tlen, B, st);
     ConvArgs f{};  // final conv (Cout = 1) + tanh on the already snake'd tensor: generic kernel
     f.x = act; f.w = tpp(ti + 1); f.bias = tpp(ti + 2); f.alpha = nullptr; f.res = nullptr; f.out = audio_out;

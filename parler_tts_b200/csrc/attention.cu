@@ -113,8 +113,7 @@ __global__ void __launch_bounds__(PRE_TC_WARPS * 32) attention_prefill_tc_kernel
 }
 
 int launch_attention(const AttnArgs& a, int dtype, cudaStream_t st, bool pdl) {
-  static const bool pre_tc = []() { const char* e = getenv("PTTS_PREFILL_ATTN_TC"); return !(e && e[0] == '0'); }();
-  if (a.q_len > 1 && dtype == PTTS_BF16 && a.nh == a.nkv && a.kv_t_stride == HD && !a.past_from_ctrl && pre_tc) {
+  if (a.q_len > 1 && dtype == PTTS_BF16 && a.nh == a.nkv && a.kv_t_stride == HD && !a.past_from_ctrl) {
     const size_t smem = 128 + (size_t)PRE_TC_WARPS * PRE_TC_WARP_BYTES;
     static bool attr_p = false;
     if (!attr_p) {

@@ -198,21 +198,23 @@ namespace ptts {
 // kernel -- both run exactly this code, hence bit-identical results.
 __device__ __forceinline__ uint32_t att_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
+// keys per ring stage
 template <typename T> struct AttChunk { static constexpr int CH = 32; };
 template <> struct AttChunk<float> { static constexpr int CH = 16; };
 
-// bytes of shared memory one warp needs (CH = keys per ring stage)
-template <typename T, int CH = AttChunk<T>::CH>
+// bytes of shared memory one warp needs
+template <typename T>
 __host__ __device__ constexpr int attn_decode_smem_per_warp() {
-  return 2 * 2 * CH * HD * (int)sizeof(T) + (3 * HD) * (int)sizeof(float);
+  return 2 * 2 * AttChunk<T>::CH * HD * (int)sizeof(T) + (3 * HD) * (int)sizeof(float);
 }
 
-template <typename T, int CH = AttChunk<T>::CH>
+template <typename T>
 __device__ __forceinline__ void attention_decode_item_warp(const AttnArgs& p, int b, int kvh, int pos, unsigned char* sm_warp, uint64_t* bars,
                                                            int lane, uint32_t& parity, int part = 0, int nparts = 1, float* xch = nullptr,
                                                            int pair_bar = 0) {
   // part / nparts: the item's cached keys are split between `nparts` warps (chunk c belongs to warp c % nparts);
   // partial (max, sum, accumulator) triples are merged through `xch` with a 64-thread named barrier `pair_bar`.
+  constexpr int CH = AttChunk<T>::CH;
   constexpr int STAGE_ELEMS = CH * HD;  // per K (or V) stage
   T* kst = reinterpret_cast<T*>(sm_warp);                   // [2][CH][64]
   T* vst = kst + 2 * STAGE_ELEMS;                            // [2][CH][64]

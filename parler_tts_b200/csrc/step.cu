@@ -135,7 +135,6 @@ struct Smem {
   long long* prof;  // CTA 0 / thread 0 timestamps of the current phase (nullptr = off)
   int pitch;
   int nbuf;
-  int dbg;
 };
 
 __device__ __forceinline__ bf16* tile_of(const Smem& sm, int buf) { return sm.tile0 + (size_t)buf * 32 * sm.pitch; }
@@ -147,7 +146,7 @@ __device__ __forceinline__ bf16* tile_of(const Smem& sm, int buf) { return sm.ti
 __device__ __forceinline__ void stage_tile(Smem& sm, int buf, const bf16* img, int M, bool mark) {
   __syncthreads();  // every generic-proxy access to the buffer (ldmatrix, reduction scratch) is done
   if (threadIdx.x == 0) {
-    if (!(sm.dbg & 8)) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // tile buffer: generic accesses (above barrier) before the async write
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // tile buffer: generic accesses (above barrier) before the async write
     const uint32_t bytes = (uint32_t)(M * sm.pitch * 2);
     mbar_expect_tx(&sm.bars[buf], bytes);
     bulk_g2s(tile_of(sm, buf), img, bytes, &sm.bars[buf]);
@@ -213,8 +212,7 @@ __device__ __forceinline__ void prefetch_kv(const StepParams& p, int l, int pos)
 }
 
 __device__ __forceinline__ void issue_prefetch(const StepParams& p, const PrefetchJob& j) {
-  if (p.dbg & 1) return;
-  if (j.kv_layer >= 0 && !(p.dbg & 2)) prefetch_kv(p, j.kv_layer, j.pos);
+  if (j.kv_layer >= 0) prefetch_kv(p, j.kv_layer, j.pos);
   if (threadIdx.x == ST_THREADS - 32) {
     if (j.w != nullptr) prefetch_slice(j.w, j.N, j.K, j.nt);
     if (j.v != nullptr) l2_prefetch(j.v, j.v_bytes);
@@ -252,7 +250,7 @@ __device__ __forceinline__ void issue_weights_thread(const StepParams& p, Smem& 
   gemm_matrix(p, ph, W, N, K, nt);
   if (task >= N / (8 * nt)) return;
   const uint32_t bytes = (uint32_t)nt * (uint32_t)K * 16u;
-  if (!(p.dbg & 4)) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
   mbar_expect_tx(&sm.bars[WBAR], bytes);
   bulk_g2s(const_cast<uint4*>(sm.wbuf), W + (size_t)task * bytes, bytes, &sm.bars[WBAR]);
 }
@@ -439,7 +437,6 @@ __global__ void __launch_bounds__(ST_THREADS, 1) decode_step_kernel(const __grid
   sm.wbuf = reinterpret_cast<const uint4*>(smem_raw + ST_HEADER + p.wbuf_offset);
   sm.pitch = H + 8;
   sm.nbuf = p.nbuf;
-  sm.dbg = p.dbg;
   sm.tile0 = reinterpret_cast<bf16*>(sm.scratch);
   sm.parity = 0;
   sm.prof = nullptr;

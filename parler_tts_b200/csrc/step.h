@@ -7,13 +7,13 @@ namespace ptts {
 
 struct StepParams {
   // shapes
-  int B, H, F, V, K, L, nh, nkv, nckv, S, P, Tmax, rope, act, qkv_rows, ckv_rows;
+  int B, H, F, V, K, L, nh, nkv, nckv, S, P, Tmax, rope, act, qkv_rows;
   float eps, scale;
   // packed weights
   const char* blob;
-  int64_t embed, pos, layer0, layer_stride, ln1_w, ln1_b, wqkv, wo, ln2_w, ln2_b, wqc, woc, ln3_w, ln3_b, fc1, fc2;
+  int64_t embed, pos, layer0, layer_stride, wqkv, wo, wqc, woc, fc1, fc2;
   int64_t c_qkv, c_qc, c_fc1, c_heads;   // folded-LayerNorm vectors
-  int64_t final_ln_w, final_ln_b, heads, rope_cos, rope_sin;
+  int64_t heads, rope_cos, rope_sin;
   // workspace
   bf16 *x, *qkv, *attn, *qc, *hbuf;  // x / attn / hbuf are tile images (row pitch H + 8; hbuf: F/H images), qkv / qc plain rows
   float* logits;
@@ -26,17 +26,12 @@ struct StepParams {
   // schedule
   int nt_qkv, nt_h, nt_fc1, nt_heads;
   int nbuf;                // activation-tile buffers (2 = double-buffered K chunks)
-  int attn_floats_per_warp;
   int64_t tile_region_bytes;   // scratch after the header: [activation tiles | weight buffer], aliased by attention
   int64_t wbuf_offset;         // weight buffer offset inside the scratch region
   int do_sample_phase;     // 1: logits -> token inside the kernel (ptts_decode_steps); 0: stop at the logits
   int sample_items;        // ceil(V / 256): logits per thread of the one-CTA-per-row sampler
   int* progress;           // debug: last phase each CTA arrived at (printed on a barrier timeout)
   int n_steps;             // cluster kernel: tokens one launch may run (stops early when every row is finished); 0 / 1 = one
-  int dbg;                 // PTTS_DBG measurement switches (bit mask, all off by default; INTEGRATION.md lists them).  step.cu: 1 no weight
-                           // L2 prefetch, 2 no K/V prefetch, 4 / 8 omit a proxy fence.  step2.cu: 1 / 2 weight / K/V L2 prefetches ON,
-                           // 16 SIMT attention, 32 acquire fence at the layer barriers, 64 release-form cluster arrive, 128 cold sampling
-                           // pass first, 256 default L2 policy for the streamed data, 512 old fc2 warp mapping
   long long* prof;         // optional [(8L+3)][8] clock64 timestamps written by CTA 0 (debug / profiles)
   // ---- cluster step kernel (step2.cu) ----
   int64_t cp[6], cp_slice[6];   // per-layer offsets / slice bytes of the (phase, cluster, rank) weight slices (layout.h)

@@ -20,8 +20,8 @@
 //     6 barriers per layer instead of 8.
 //   * weights: one contiguous slice per (phase, cluster, rank) (layout.h cpack, built once by ptts_decoder_finalize), streamed by
 //     ONE bulk copy per job into a 2 x 64 KB ring two jobs ahead, with an L2 evict-first policy like the K/V rows (1.2 GB per token
-//     must not evict the kernel's own instructions and the small reused tensors).  HBM -> L2 prefetches a layer ahead exist behind
-//     PTTS_DBG=1/2 and measured slower (profiles/r02_step2_phases.md).
+//     must not evict the kernel's own instructions and the small reused tensors).  No HBM -> L2 prefetches a layer ahead: they
+//     measured slower (profiles/r02_step2_phases.md).
 //   * fc2 (one n-tile per destination, K slice F/4): every warp takes all four n-tiles over an eighth of the K slice, the partial
 //     tiles are added inside the CTA and one block per destination crosses the cluster (A fragments read once per CTA).
 //   * the activation slice of the next phase is requested by the barrier's polling thread the moment the barrier opens; the
@@ -46,7 +46,6 @@ constexpr int C = 4;            // CTAs per cluster
 constexpr int V = 8;            // virtual ranks = warps per CTA: warp w reduces K-half (w >> 2) for destination rank (w & 3)
 constexpr int THREADS = 256;
 constexpr int ROWS = 32;        // batch rows (two m16 tiles; the head phases work on one half = one m16 tile)
-constexpr int ATT_CH = 16;      // keys per K/V ring stage of an attention warp
 constexpr int PROF_STRIDE = 16;  // clock64 stamps per phase row of the optional profile buffer (tools/profile_step2.py)
 constexpr int QMAX = 6;         // n-tiles per warp (QKV: 24 n-tiles of a head over 4 destination groups)
 constexpr int OFF_STATS = 256, OFF_PART = 512, OFF_RES = 2560, OFF_CVEC = 3584;
@@ -102,22 +101,9 @@ __device__ __forceinline__ void cluster_wait() { asm volatile("barrier.cluster.w
 // The per-phase cluster barrier only guards buffer REUSE (a peer may overwrite my receive slots / I may overwrite a send block once
 // everyone has consumed the previous phase's); the data itself is ordered by the exchange mbarrier.  A write-after-read needs no
 // release: the default .release arrive is a gpu-scope MEMBAR per warp (it waits for the epilogue's global stores to be acknowledged,
-// ~0.5 us, a second time before the layer barrier does).  PTTS_DBG=64 restores the release form for A/B runs.
-__device__ __forceinline__ void cluster_arrive_reuse(bool release) {
-  if (release) asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  else asm volatile("barrier.cluster.arrive.relaxed.aligned;" ::: "memory");
-}
+// ~0.5 us, a second time before the layer barrier does).
+__device__ __forceinline__ void cluster_arrive_reuse() { asm volatile("barrier.cluster.arrive.relaxed.aligned;" ::: "memory"); }
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void l2_prefetch(const void* p, uint32_t bytes, bool on = true) {
-  if (!on) return;
-  const char* c = reinterpret_cast<const char*>(p);
-  while (bytes > 0) {
-    const uint32_t n = bytes > 32768u ? 32768u : bytes;
-    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(c), "r"(n) : "memory");
-    c += n;
-    bytes -= n;
-  }
-}
 __device__ __forceinline__ unsigned ld_relaxed(const unsigned* p) { unsigned v; asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory"); return v; }
 __device__ __forceinline__ void red_release_add(unsigned* p, unsigned v) { asm volatile("red.release.gpu.global.add.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory"); }
 __device__ __forceinline__ void ldsm4(uint32_t (&r)[4], const void* smem_ptr) {
@@ -127,9 +113,8 @@ __device__ __forceinline__ void prof_mark(long long* prof, int slot) { if (prof 
 
 // ---- device-wide barrier (same protocol as step.cu) -----------------------------------------------
 // `post` runs on thread 0 the moment the barrier opens (before the CTA is released): the next phase's activation copy.
-// `side` runs on thread 32 while thread 0 polls.
-template <typename Post, typename Side>
-__device__ __forceinline__ unsigned grid_sync(unsigned* ctr, unsigned target, int ph, Post post, Side side, bool acq_fence = true) {
+template <typename Post>
+__device__ __forceinline__ unsigned grid_sync(unsigned* ctr, unsigned target, int ph, Post post, bool acq_fence = true) {
   target += gridDim.x;
   asm volatile("fence.proxy.async.global;" ::: "memory");  // this thread's global writes -> other CTAs' TMA reads (writer side)
   __syncthreads();
@@ -141,11 +126,9 @@ __device__ __forceinline__ unsigned grid_sync(unsigned* ctr, unsigned target, in
     }
     // Everything this kernel reads that another CTA wrote during the same launch goes through L2 (TMA bulk copies of the images
     // and the K/V rows, __ldcg of the logits / EOS columns), so the L1 invalidation of an acquire fence protects nothing here and
-    // costs 0.4 us per barrier (profiles/r02_step2_phases.md): the per-layer barriers skip it, PTTS_DBG=32 puts it back.
+    // costs 0.4 us per barrier (profiles/r02_step2_phases.md): the per-layer barriers skip it.
     if (acq_fence) asm volatile("fence.acq_rel.gpu;" ::: "memory");
     post();
-  } else if (threadIdx.x == 32) {
-    side();
   }
   __syncthreads();
   return target;
@@ -158,7 +141,7 @@ __device__ __forceinline__ unsigned grid_sync(unsigned* ctr, unsigned target, in
 // 6 extra MMAs per k-tile and m-tile buy an exchange without any CTA-wide synchronisation).
 template <int QN, int MT, int SETS, bool STATS>
 __device__ __forceinline__ void mma_slice(float (&out)[2][6][4], RowStatFrag& rst, const bf16* xs, int apitch, const uint4* wb, int KT, int kt_lo,
-                                          int kt_hi, int dgrp, int lrow, int lcol) {
+                                          int kt_hi, int lrow, int lcol) {
   float acc[SETS][MT][QN][4];
 #pragma unroll
   for (int s = 0; s < SETS; s++)
@@ -270,12 +253,9 @@ __global__ void __launch_bounds__(THREADS, 1) decode_step_cluster_kernel(const _
   }
   attention_decode_init_warp(attbars + 2 * warp, lane);
   cluster_arrive(); cluster_wait();   // every peer's mbarriers exist before any remote complete_tx
-  // HBM -> L2 prefetches a layer ahead cost more than they bring here (1097 -> 1070 us per step without them: the shared-memory
-  // ring already runs two jobs = ~8 us ahead of its consumer, and every cp.async.bulk.prefetch.L2 is ~100 cycles of issue time
-  // inside a phase): off by default, PTTS_DBG=1 switches them on (profiles/r02_step2_phases.md)
-  const bool pf_on = (p.dbg & 1) != 0;   // PTTS_DBG=1: weight / folded-LN L2 prefetches on
-  const bool pf_kv = (p.dbg & 2) != 0;   // PTTS_DBG=2: next layer's K/V rows -> L2 during the out-proj phases
-  const bool acq = (p.dbg & 32) != 0;   // PTTS_DBG=32: put the acquire fence back (grid_sync explains why it is not needed)
+  // No HBM -> L2 prefetches a layer ahead: they cost more than they bring here (1097 -> 1070 us per step without them: the
+  // shared-memory ring already runs two jobs = ~8 us ahead of its consumer, and every cp.async.bulk.prefetch.L2 is ~100 cycles of
+  // issue time inside a phase; profiles/r02_step2_phases.md)
   unsigned* const bar_ctr = p.bar + (gen & 1u);
   unsigned bar_target = 0u;
   if (cta == 0 && tid == 0) p.bar[(gen + 1u) & 1u] = 0u;  // the counter the NEXT launch will use
@@ -294,21 +274,7 @@ __global__ void __launch_bounds__(THREADS, 1) decode_step_cluster_kernel(const _
     // in flight (it cost ~0.5 us wherever one sat behind a 64 KB weight copy).  The one generic-written corner (the attention
     // merge scratch of the q_cross phase) is covered by the fence thread 0 executes at every device-wide barrier (request_slice).
     mbar_expect_tx(&wbar[j & 1], bytes);
-    if (p.dbg & 256) bulk_g2s(smem + HDR + (j & 1) * WB_BYTES, src, bytes, &wbar[j & 1]);   // (A/B: default L2 policy)
-    else bulk_g2s_stream(smem + HDR + (j & 1) * WB_BYTES, src, bytes, &wbar[j & 1]);
-  };
-  // the same requests cut into one piece per warp (issued by lane 0 of every warp: a prefetch is ~100 cycles of issue time)
-  auto prefetch_weight_job_part = [&](int j, int w) {
-    const char* src; uint32_t bytes;
-    if (pf_on && weight_job(p, j, cta, rank, src, bytes)) { const uint32_t pc = (bytes / V) & ~15u; l2_prefetch(src + (size_t)w * pc, w == V - 1 ? bytes - (V - 1) * pc : pc); }
-  };
-  auto prefetch_kv_part = [&](int l, bool cross, int w) {  // warp w: item w >> 1, K (even w) or V (odd w)
-    const int T = cross ? p.S : p.Tmax, n = cross ? p.S : pos;
-    const int b = 16 * half + 4 * rank + (w >> 1);
-    if (!pf_kv || n <= 0 || b >= B) return;
-    const char* kc = cross ? p.cross_kv + p.cross_layer_stride * l : p.self_kv + p.self_layer_stride * l;
-    const char* k = kc + ((size_t)b * p.nh + head) * T * HD * 2 + ((w & 1) ? (size_t)B * p.nh * T * HD * 2 : 0);
-    l2_prefetch(k, (uint32_t)(n * HD * 2));
+    bulk_g2s_stream(smem + HDR + (j & 1) * WB_BYTES, src, bytes, &wbar[j & 1]);
   };
   // ---- one launch runs up to p.n_steps tokens (ptts_decode_steps): the ~10 us between dependent cooperative launches, the launch
   // skew in front of the first barrier and the cold instruction fetches of the once-per-token phases are paid once per launch.
@@ -320,12 +286,8 @@ __global__ void __launch_bounds__(THREADS, 1) decode_step_cluster_kernel(const _
   for (int it = 0; it < n_steps; it++) {
   pos = p.P + cur_len - 1;
   prof = prof0;
-  cluster_arrive_reuse(false);        // pre-arm: pairs with the first phase's "exchange buffers free" wait
+  cluster_arrive_reuse();        // pre-arm: pairs with the first phase's "exchange buffers free" wait
   if (tid == 0) { issue_weight_job(0); issue_weight_job(1); }
-  if (lane == 0) {
-    for (int j = 2; j < JOBS_PER_LAYER; j++) prefetch_weight_job_part(j, warp);
-    prefetch_kv_part(0, false, warp); prefetch_kv_part(0, true, warp);
-  }
 
   // global activation images, K-sliced for their consumer: [4 slices][32 rows][slice width + 8] bf16
   bf16* const x_img = p.cl_x;       // slices of H/4 columns (consumers: QKV, q_cross, fc1, lm heads)
@@ -370,7 +332,7 @@ __global__ void __launch_bounds__(THREADS, 1) decode_step_cluster_kernel(const _
   {
     const bf16* nimg; uint32_t nbytes;
     slice_of(PH_QKV, nimg, nbytes);
-    bar_target = grid_sync(bar_ctr, bar_target, -1, [&]() { request_slice(nimg, nbytes); }, []() {}, acq);
+    bar_target = grid_sync(bar_ctr, bar_target, -1, [&]() { request_slice(nimg, nbytes); }, false);
   }
   prof_mark(prof, 7);
 
@@ -408,7 +370,7 @@ __global__ void __launch_bounds__(THREADS, 1) decode_step_cluster_kernel(const _
     // fragments -- 512 B of shared memory per HMMA, 262 KB per phase, and the shared-memory port (128 B/clk), not the tensor pipe,
     // sets the 1.5 us.  Instead every warp takes ALL four n-tiles over an eighth of the K slice (A read once per CTA); the eight
     // partial tiles are added inside the CTA (shared memory, fixed order) and ONE block per destination crosses the cluster.
-    const bool fc2_wide = (sub == PH_FC2) && q == 1 && (KT & 7) == 0 && !(p.dbg & 512);
+    const bool fc2_wide = (sub == PH_FC2) && q == 1 && (KT & 7) == 0;
 
     // folded-LayerNorm vectors of this phase's features: requested now, parked in shared memory after the MMA loop (a global
     // load followed at once by its shared-memory store would park the warp for an L2 round trip in front of the MMAs)
@@ -447,31 +409,20 @@ __global__ void __launch_bounds__(THREADS, 1) decode_step_cluster_kernel(const _
       const int nt0 = (sub == PH_QKV) ? (dgrp & 1) * q : dgrp * q;   // first n-tile of this warp inside that job's slice
       const uint4* wb = reinterpret_cast<const uint4*>(smem + HDR + (wjob & 1) * WB_BYTES) + (size_t)nt0 * KT * 32 + lane;
       const int kt_lo = kh * (KT >> 1), kt_hi = kt_lo + (KT >> 1);
-      if (sub == PH_QKV) mma_slice<6, 1, 1, true>(acc, rst, xs, apitch, wb, KT, kt_lo, kt_hi, dgrp, lrow, lcol);
-      else if (sub == PH_QC) mma_slice<2, 1, 4, true>(acc, rst, xs, apitch, wb, KT, kt_lo, kt_hi, dgrp, lrow, lcol);
+      if (sub == PH_QKV) mma_slice<6, 1, 1, true>(acc, rst, xs, apitch, wb, KT, kt_lo, kt_hi, lrow, lcol);
+      else if (sub == PH_QC) mma_slice<2, 1, 4, true>(acc, rst, xs, apitch, wb, KT, kt_lo, kt_hi, lrow, lcol);
       else if (sub == PH_FC1) {
-        if (q == 4) mma_slice<4, 2, 1, true>(acc, rst, xs, apitch, wb, KT, kt_lo, kt_hi, dgrp, lrow, lcol);
-        else if (q == 2) mma_slice<2, 2, 2, true>(acc, rst, xs, apitch, wb, KT, kt_lo, kt_hi, dgrp, lrow, lcol);
-        else mma_slice<1, 2, 4, true>(acc, rst, xs, apitch, wb, KT, kt_lo, kt_hi, dgrp, lrow, lcol);
+        if (q == 4) mma_slice<4, 2, 1, true>(acc, rst, xs, apitch, wb, KT, kt_lo, kt_hi, lrow, lcol);
+        else if (q == 2) mma_slice<2, 2, 2, true>(acc, rst, xs, apitch, wb, KT, kt_lo, kt_hi, lrow, lcol);
+        else mma_slice<1, 2, 4, true>(acc, rst, xs, apitch, wb, KT, kt_lo, kt_hi, lrow, lcol);
       } else if (fc2_wide) {
         const uint4* wall = reinterpret_cast<const uint4*>(smem + HDR + (j0 & 1) * WB_BYTES) + lane;   // all four n-tiles
-        mma_slice<4, 2, 1, false>(acc, rst, xs, apitch, wall, KT, warp * (KT >> 3), (warp + 1) * (KT >> 3), 0, lrow, lcol);
-      } else mma_slice<1, 2, 4, false>(acc, rst, xs, apitch, wb, KT, kt_lo, kt_hi, dgrp, lrow, lcol);
+        mma_slice<4, 2, 1, false>(acc, rst, xs, apitch, wall, KT, warp * (KT >> 3), (warp + 1) * (KT >> 3), lrow, lcol);
+      } else mma_slice<1, 2, 4, false>(acc, rst, xs, apitch, wb, KT, kt_lo, kt_hi, lrow, lcol);
     }
     prof_mark(prof, 2);
     if (has_ln && tid < (rowpart ? Nc : 8 * q)) { cvec[tid] = cv1; cvec[256 + tid] = cv2; }   // read in the epilogue, several barriers later
     __syncthreads();  // activation slice and weight buffer(s) are dead
-    if (lane == 0 && (pf_on || pf_kv)) {  // asynchronous requests, one or two per warp so that no single thread holds the CTA back
-      for (int i = 0; i < njobs; i++) prefetch_weight_job_part(j0 + i + JOBS_PER_LAYER, warp);  // same job, next layer (or lm heads) -> L2
-      if (sub == PH_QKV && warp == 2 && l + 1 < p.L) {   // next layer's folded-LN vectors: every CTA pulls a 1/grid share into L2
-        const int64_t c_bytes = p.c_fc1 + (int64_t)2 * F * 4 - p.c_qkv;
-        const uint32_t share = (uint32_t)(((c_bytes / (int)gridDim.x) + 15) & ~15);
-        const int64_t o = (int64_t)cta * share;
-        if (pf_on && o < c_bytes) l2_prefetch(lb + p.layer_stride + p.c_qkv + o, (uint32_t)(c_bytes - o < share ? c_bytes - o : share));
-      }
-      if (sub == PH_O && l + 1 < p.L) prefetch_kv_part(l + 1, false, warp);
-      if (sub == PH_OC && l + 1 < p.L) prefetch_kv_part(l + 1, true, warp);
-    }
     prof_mark(prof, 12);
     cluster_wait();  // every peer is past its previous epilogue: my send blocks have been read, its receive slots are free
     prof_mark(prof, 13);
@@ -517,7 +468,6 @@ __global__ void __launch_bounds__(THREADS, 1) decode_step_cluster_kernel(const _
       }
     } else {
       unsigned char* mine = send + (size_t)warp * wsend;
-      const bool merged = rowpart && !(p.dbg & 1024);
       if (!rowpart) {
         float* bp = reinterpret_cast<float*>(mine + 256);
 #pragma unroll
@@ -549,8 +499,8 @@ __global__ void __launch_bounds__(THREADS, 1) decode_step_cluster_kernel(const _
           const int row = g + 8 * hh;
           // block of destination rank d = row >> 2: [destination][warp] order, so that ONE copy per destination ships all eight warps'
           // blocks (a bulk copy costs ~0.1 us of issue time through the uniform datapath: 4 per warp were 0.4 us of every warp's
-          // critical path; PTTS_DBG=1024 keeps the per-warp copies, [warp][destination] order)
-          unsigned char* blk_d = merged ? send + ((size_t)(row >> 2) * V + warp) * blk : mine + (size_t)(row >> 2) * blk;
+          // critical path)
+          unsigned char* blk_d = send + ((size_t)(row >> 2) * V + warp) * blk;
           float* bp = reinterpret_cast<float*>(blk_d + 32) + (row & 3) * qc + 2 * t4;
 #pragma unroll
           for (int j = 0; j < QMAX; j++)
@@ -567,15 +517,12 @@ __global__ void __launch_bounds__(THREADS, 1) decode_step_cluster_kernel(const _
           fence_proxy_async_smem();
           bulk_s2peer(mapa(s32(recv + (size_t)(2 * rank + kh) * blk), (uint32_t)dgrp), mine, (uint32_t)blk, mapa(s32(xbar), (uint32_t)dgrp));
         }
-      } else if (merged) {
+      } else {
         __syncthreads();   // all eight warps' blocks are staged
         if (warp < C && lane == 0) {   // warp d ships [d][0..7] to rank d: it lands as slots 8 rank .. 8 rank + 7 there
           fence_proxy_async_smem();
           bulk_s2peer(mapa(s32(recv + (size_t)(8 * rank) * blk), (uint32_t)warp), send + (size_t)warp * V * blk, (uint32_t)(V * blk), mapa(s32(xbar), (uint32_t)warp));
         }
-      } else if (lane < C) {
-        fence_proxy_async_smem();
-        bulk_s2peer(mapa(s32(recv + (size_t)(8 * rank + warp) * blk), (uint32_t)lane), mine + (size_t)lane * blk, (uint32_t)blk, mapa(s32(xbar), (uint32_t)lane));
       }
     }
     // Requests that are not on the critical path go out now, while the partial sums travel: the weight ring's refill (two jobs
@@ -627,7 +574,7 @@ __global__ void __launch_bounds__(THREADS, 1) decode_step_cluster_kernel(const _
         att_xch = reinterpret_cast<float*>(bD + 32768) + (warp >> 1) * 128;
       }
       att_f = reinterpret_cast<float*>(Rg + 65536) + warp * 192;   // query / new key / new value: a corner of R the exchange never uses
-      if (att_b < B && !(p.dbg & 16)) attention_tc_issue_first(item, att_ring, attbars + 2 * warp, lane, warp & 1, 2, !(p.dbg & 256));
+      if (att_b < B) attention_tc_issue_first(item, att_ring, attbars + 2 * warp, lane, warp & 1, 2, true);
     }
     prof_mark(prof, 15);
     mbar_wait(xbar, par_x, 2);
@@ -715,50 +662,13 @@ __global__ void __launch_bounds__(THREADS, 1) decode_step_cluster_kernel(const _
     }
     prof_mark(prof, 4);
     __syncthreads();   // this CTA's receive slots are consumed (and q|k|v complete): peers may send the next phase's partials
-    cluster_arrive_reuse((p.dbg & 64) != 0);
-    if (rowpart && (p.dbg & 16)) {
-      // the SIMT attention's scratch aliases the send blocks: the peers must have RECEIVED them (each is past its exchange wait) first
-      cluster_wait();
-      cluster_arrive();  // re-arm for the next phase's "exchange buffers free" wait
-    }
+    cluster_arrive_reuse();
 
     // ---- attention of this rank's 4 (row, head) items: two warps per item (first two K/V stages were requested after the MMA) ----
     if (rowpart) {
-      if (att_b < B) {
-        if (p.dbg & 16) {  // A/B: the SIMT sweep (its ring layout: K/V stages then 192 floats, inside the R region)
-          AttnArgs att{};
-          att.ctrl = nullptr; att.B = B; att.nh = p.nh; att.nkv = p.nh; att.q_len = 1;
-          att.past_from_ctrl = 0; att.past_len = pos; att.prefix = p.P;
-          att.rope = p.rope; att.rope_cos = blob + p.rope_cos; att.rope_sin = blob + p.rope_sin; att.scale = p.scale;
-          const bf16* qkv_s = reinterpret_cast<const bf16*>(Rg + QKV_OFF);
-          const int row_base = 16 * half + 4 * rank;
-          const bf16* qbase = qkv_s - (size_t)row_base * Nc - (size_t)head * HD;
-          att.q = qbase; att.ldq = Nc; att.q_col0 = 0;
-          att.ldo = pitch;
-          att.out = a_img + (size_t)(head >> 2) * x_slice_elems + (head & 3) * HD - (size_t)head * HD;
-          if (sub == PH_QKV) {
-            att.knew = qbase; att.vnew = qbase; att.ldkv = Nc; att.k_col0 = HD; att.v_col0 = 2 * HD;
-            char* kc = p.self_kv + p.self_layer_stride * l;
-            att.kcache = kc; att.vcache = kc + (size_t)B * p.nh * p.Tmax * HD * 2;
-            att.kv_b_stride = (int64_t)p.nh * p.Tmax * HD; att.kv_h_stride = (int64_t)p.Tmax * HD; att.kv_t_stride = HD;
-            att.key_mask = p.prompt_mask; att.mask_len = p.P; att.mask_ld = p.P;
-            att.cross = 0; att.kv_len = 0; att.kv_capacity = p.Tmax;
-          } else {
-            att.knew = nullptr; att.vnew = nullptr;
-            char* ck = p.cross_kv + p.cross_layer_stride * l;
-            att.kcache = ck; att.vcache = ck + (size_t)B * p.nh * p.S * HD * 2;
-            att.kv_b_stride = (int64_t)p.nh * p.S * HD; att.kv_h_stride = (int64_t)p.S * HD; att.kv_t_stride = HD;
-            att.key_mask = p.enc_mask; att.mask_len = p.S; att.mask_ld = p.S;
-            att.cross = 1; att.kv_len = p.S; att.kv_capacity = p.S;
-          }
-          unsigned char* region = Rg + (size_t)warp * attn_decode_smem_per_warp<bf16, ATT_CH>();
-          float* xr = reinterpret_cast<float*>(Rg + 73728) + (warp >> 1) * 128;
-          attention_decode_item_warp<bf16, ATT_CH>(att, att_b, head, pos, region, attbars + 2 * warp, lane, att_parity, warp & 1, 2, xr, (warp >> 1) + 1);
-        } else {
-          attention_decode_item_warp_tc(item, att_ring, att_ring1, att_f, attbars + 2 * warp, lane, att_parity, warp & 1, 2, att_xch,
-                                        (warp >> 1) + 1, warp == 0 ? prof : nullptr, true, !(p.dbg & 256));
-        }
-      }
+      if (att_b < B)
+        attention_decode_item_warp_tc(item, att_ring, att_ring1, att_f, attbars + 2 * warp, lane, att_parity, warp & 1, 2, att_xch,
+                                      (warp >> 1) + 1, warp == 0 ? prof : nullptr, true, true);
       prof_mark(prof, 5);
       if (sub == PH_QC) {   // fc1's weights were held back: the K/V rings used their buffer
         __syncthreads();
@@ -777,7 +687,7 @@ __global__ void __launch_bounds__(THREADS, 1) decode_step_cluster_kernel(const _
     const bf16* nimg; uint32_t nbytes;
     if (last) { nimg = x_img; nbytes = (uint32_t)(C * x_slice_elems * 2); }   // lm heads: the whole x image
     else slice_of((sub + 1) % 6, nimg, nbytes);
-    bar_target = grid_sync(bar_ctr, bar_target, ph, [&]() { request_slice(nimg, nbytes); }, []() {}, acq);
+    bar_target = grid_sync(bar_ctr, bar_target, ph, [&]() { request_slice(nimg, nbytes); }, false);
     prof_mark(prof, 7);
   }
   cluster_wait();  // balance the last phase's arrive
@@ -789,9 +699,6 @@ __global__ void __launch_bounds__(THREADS, 1) decode_step_cluster_kernel(const _
     const int ntasks = p.K * p.V / 32;
     const float* c1 = reinterpret_cast<const float*>(blob + p.c_heads);
     const float* c2 = c1 + p.K * p.V;
-    if (lane == 0) {  // layer 0 of the NEXT token -> L2 (the cache outlives the kernel): its first phases start warm
-      for (int j = 0; j < JOBS_PER_LAYER; j++) prefetch_weight_job_part(j, warp);
-    }
     mbar_wait(abar, par_a, 3);
     par_a ^= 1u;
     const bf16* xs = reinterpret_cast<const bf16*>(Rg);   // [4 slices][32][pitch]
@@ -871,24 +778,21 @@ __global__ void __launch_bounds__(THREADS, 1) decode_step_cluster_kernel(const _
     }
   }
   prof_mark(prof, 6);
-  bar_target = grid_sync(bar_ctr, bar_target, n_phases, []() {}, []() {});
+  bar_target = grid_sync(bar_ctr, bar_target, n_phases, []() {});
   prof = prof0 ? prof0 + (size_t)(n_phases + 2) * PROF_STRIDE : nullptr;  // tail row: sampling / barrier
   prof_mark(prof, 0);
   if (p.do_sample_phase) {
     const ptts_gen_params gp = *p.sa.gen;
     const int BK = B * p.K;
-    // PTTS_DBG=128 (measurement only): a first, cold pass (instruction fetch) before the stamped one; the pass is idempotent
-    for (int pass = (p.dbg & 128) ? 0 : 1; pass < 2; pass++) {
-      sample_all_rows_cta<ITEMS>(p.sa, gp, cta, (int)gridDim.x, BK, cur_len);
-      prof_mark(prof, pass == 0 ? 4 : 1);
-    }
+    sample_all_rows_cta<ITEMS>(p.sa, gp, cta, (int)gridDim.x, BK, cur_len);
+    prof_mark(prof, 1);
     // every CTA learns whether any row is still unfinished: thread 0 reads the counter the moment the barrier opens (after its
     // acquire fence); the counter is reset only when the launch ends, so a step's count is the growth since the previous step
     bar_target = grid_sync(bar_ctr, bar_target, n_phases + 1, [&]() {
       const int tot = *reinterpret_cast<volatile int*>(&ctrl->n_unfinished);
       s_next_active = (tot - unfinished_prev > 0) ? 1 : 0;
       unfinished_prev = tot;
-    }, []() {});
+    });
     prof_mark(prof, 2);
   }
   bool go_on = false;

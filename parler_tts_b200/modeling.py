@@ -529,7 +529,7 @@ class ParlerTTSForConditionalGeneration:
         input_ids = input_ids.to(self.device)
         attention_mask = None if attention_mask is None else attention_mask.to(self.device)
         if not hasattr(self, "_enc_graphs"):
-            self._enc_graphs, self._enc_graph_ok = {}, os.environ.get("PTTS_ENCODER_GRAPH", "1") != "0"
+            self._enc_graphs, self._enc_graph_ok = {}, True
         if not self._enc_graph_ok or self.device.type != "cuda":
             return self._encode_text_eager(input_ids, attention_mask)
         key = (tuple(input_ids.shape), attention_mask is not None)

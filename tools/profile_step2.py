@@ -74,7 +74,5 @@ r0, rh, rt = t[0], t[nph + 1], t[nph + 2]
 print(f"prologue {us(r0[0] - rt[3]):.2f} | embed {us(r0[6] - r0[0]):.2f} + barrier {us(r0[7] - r0[6]):.2f} | lm heads {us(rh[6] - rh[0]):.2f} "
       f"(tile + stats {us(rh[1] - rh[0]):.2f}) | barrier {us(rt[0] - rh[6]):.2f} | sampling {us(rt[1] - rt[0]):.2f} | last barrier {us(rt[2] - rt[1]):.2f} "
       f"| kernel span {us(rt[2] - rt[3]):.1f} us")
-if rt[4] > 0:
-    print(f"PTTS_DBG=128: cold sampling pass {us(rt[4] - rt[0]):.2f} us, second (warm) pass {us(rt[1] - rt[4]):.2f} us")
 os.makedirs("gpurun_out", exist_ok=True)
 json.dump({"step_us": e0.elapsed_time(e1) * 1e3, "phases_us": out}, open("gpurun_out/step2_phases.json", "w"), indent=1)
