@@ -114,12 +114,19 @@ int ptts_decoder_finalize(const ptts_decoder_config* cfg, void* blob, void* stre
  * self-attention cache of max_cache_len positions (>= P + max_length - 1). */
 int ptts_workspace_bytes(const ptts_decoder_config* cfg, int32_t B, int32_t P, int32_t S,
                          int32_t max_cache_len, int64_t* out_bytes);
+/* Same, for a session whose first forward may take up to max_prefix (>= 1) decoder columns (ptts_prefill_ids: a
+ * voice-prompt prefix, modeling_parler_tts.py:3136-3194).  ptts_workspace_bytes is the max_prefix = 1 case. */
+int ptts_workspace_bytes_ex(const ptts_decoder_config* cfg, int32_t B, int32_t P, int32_t S,
+                            int32_t max_cache_len, int32_t max_prefix, int64_t* out_bytes);
 
 typedef struct ptts_session ptts_session; /* host-side object: pointers into blob/workspace + CUDA graphs */
 
 int ptts_session_create(const ptts_decoder_config* cfg, const void* blob, void* workspace,
                         int64_t workspace_bytes, int32_t B, int32_t P, int32_t S, int32_t max_cache_len,
                         ptts_session** out);
+int ptts_session_create_ex(const ptts_decoder_config* cfg, const void* blob, void* workspace,
+                           int64_t workspace_bytes, int32_t B, int32_t P, int32_t S, int32_t max_cache_len,
+                           int32_t max_prefix, ptts_session** out);
 int ptts_session_destroy(ptts_session* s);
 
 /* Start a generate() call: reset per-call state (ids history = BOS column, processor state,
@@ -137,6 +144,13 @@ int ptts_generate_begin(ptts_session* s, const ptts_gen_params* gen, void* strea
  *   enc_mask      [B, S] int64 or NULL                              (attention_mask)            */
 int ptts_prefill(ptts_session* s, const void* prompt_hidden, const int64_t* prompt_mask,
                  const void* enc_hidden, const int64_t* enc_mask, void* stream);
+/* Prefill over n decoder columns (voice-prompt continuation, :3017-3044, :3523-3528): prompt prefix + prefix_ids
+ * [B*K, n] int64 (already delay-patterned, column 0 = BOS) in one forward of q_len = P + n; writes raw_ids[:, :n], sets the
+ * device cur_len = n and leaves the logits of the last position.  1 <= n <= the session's max_prefix, n < max_length.
+ * ptts_prefill is the n = 1 case with the BOS column ptts_generate_begin staged. */
+int ptts_prefill_ids(ptts_session* s, const void* prompt_hidden, const int64_t* prompt_mask,
+                     const void* enc_hidden, const int64_t* enc_mask, const int64_t* prefix_ids, int32_t n,
+                     void* stream);
 
 /* One cached decode step for the ids currently staged in the workspace (the delay-masked last
  * column).  Leaves f32 logits [B*K, V] in the workspace.  Replaces prepare_inputs_for_generation
@@ -147,7 +161,8 @@ int ptts_decode_forward(ptts_session* s, void* stream);
  * (logits_processors.py:44-53), temperature/top-k/top-p, softmax + sampling or argmax, finished-row
  * padding, history append, EOS/max-length stopping, delay-mask override of the next input.
  * Replaces one iteration of GenerationMixin._sample (transformers 4.46.1) + :2909.
- * forced_tokens: NULL, or [B*K] int64 device tokens that replace the drawn ones (teacher forcing). */
+ * forced_tokens: NULL, or [B*K] int64 device tokens that replace the drawn ones (teacher forcing); a negative entry
+ * means "draw this row" (the prompt codes the delay pattern puts after a voice-prompt prefix are forced per row). */
 int ptts_sample(ptts_session* s, const int64_t* forced_tokens, void* stream);
 
 /* n_steps x (ptts_decode_forward + ptts_sample), replayed from a CUDA graph, no host sync.
@@ -205,6 +220,34 @@ int ptts_dac_workspace_bytes(const ptts_dac_config* cfg, int32_t B, int32_t T, i
  * audio [B, 1, hop*T] in cfg->dtype.  = quantizer.from_codes (:138) + model.decode (:139). */
 int ptts_dac_decode(const ptts_dac_config* cfg, const void* blob, void* workspace, int64_t workspace_bytes,
                     const int64_t* codes, int32_t B, int32_t T, void* audio_out, void* stream);
+
+/* ---- DAC encode (voice prompt) ------------------------------------------------------------- */
+/* Separate from ptts_dac_config so that the decode ABI and the decode blob keep their layout.  Shapes per
+ * transformers' DacEncoder / DacResidualVectorQuantizer (models/dac/modeling_dac.py:442-473, :281-343). */
+typedef struct ptts_dac_encoder_config {
+  int32_t encoder_dim;         /* 64: conv1 width; block i runs at encoder_dim << i channels, outputs encoder_dim << (i+1) */
+  int32_t n_blocks;            /* 4 */
+  int32_t strides[8];          /* 2,4,8,8 (even) */
+  int32_t latent_dim;          /* 1024 */
+  int32_t n_codebooks, codebook_size, codebook_dim;
+  int32_t dtype;               /* PTTS_BF16 or PTTS_F32 */
+} ptts_dac_encoder_config;
+
+int ptts_dac_encoder_blob_bytes(const ptts_dac_encoder_config* cfg, int64_t* out_bytes);
+int ptts_dac_encoder_num_tensors(const ptts_dac_encoder_config* cfg, int32_t* out);
+/* Pack one weight-norm-folded tensor; see parler_tts_b200/dac_wrapper.py::_dac_encoder_tensor_list for the
+ * (id -> state-dict key) table.  Packing a codebook also stores its L2-normalised copy for the code search. */
+int ptts_dac_encoder_pack(const ptts_dac_encoder_config* cfg, void* blob, int32_t name_id, const void* src,
+                          int32_t src_dtype, int64_t numel, void* stream);
+int ptts_dac_encoder_workspace_bytes(const ptts_dac_encoder_config* cfg, int32_t B, int64_t n_samples, int64_t* out_bytes);
+/* DACModel.encode (dac_wrapper/modeling_dac.py:33-104) = DAC.encode: encoder network + residual vector quantizer.
+ *   audio     [B][n_samples] cfg->dtype, already right-padded to a multiple of the hop (prod(strides))
+ *   codes_out [B][n_q][n_samples / hop] int64 (n_q in 1..n_codebooks)
+ *   z_out     [B][n_samples / hop][latent_dim] cfg->dtype, the quantized latent (sum of the n_q codebooks'
+ *             out_proj outputs); NULL = not written */
+int ptts_dac_encode(const ptts_dac_encoder_config* cfg, const void* blob, void* workspace, int64_t workspace_bytes,
+                    const void* audio, int32_t B, int64_t n_samples, int32_t n_q, int64_t* codes_out, void* z_out,
+                    void* stream);
 
 #ifdef __cplusplus
 }

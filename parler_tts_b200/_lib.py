@@ -39,6 +39,11 @@ class DacConfigC(C.Structure):
                 ("strides", C.c_int32 * 8), ("dtype", C.c_int32)]
 
 
+class DacEncoderConfigC(C.Structure):
+    _fields_ = [("encoder_dim", C.c_int32), ("n_blocks", C.c_int32), ("strides", C.c_int32 * 8), ("latent_dim", C.c_int32),
+                ("n_codebooks", C.c_int32), ("codebook_size", C.c_int32), ("codebook_dim", C.c_int32), ("dtype", C.c_int32)]
+
+
 # tensor ids (include/ptts_b200.h)
 T_EMBED_TOKENS, T_POS_TABLE, T_LN1_W, T_LN1_B, T_SELF_Q, T_SELF_K, T_SELF_V, T_SELF_O = range(8)
 T_LN2_W, T_LN2_B, T_CROSS_Q, T_CROSS_K, T_CROSS_V, T_CROSS_O, T_LN3_W, T_LN3_B = range(8, 16)
@@ -53,6 +58,9 @@ _SIGS = {
     "ptts_decoder_finalize": (C.c_int, [C.POINTER(DecoderConfigC), _VP, _VP]),
     "ptts_workspace_bytes": (C.c_int, [C.POINTER(DecoderConfigC), _I32, _I32, _I32, _I32, C.POINTER(_I64)]),
     "ptts_session_create": (C.c_int, [C.POINTER(DecoderConfigC), _VP, _VP, _I64, _I32, _I32, _I32, _I32, C.POINTER(_VP)]),
+    "ptts_workspace_bytes_ex": (C.c_int, [C.POINTER(DecoderConfigC), _I32, _I32, _I32, _I32, _I32, C.POINTER(_I64)]),
+    "ptts_session_create_ex": (C.c_int, [C.POINTER(DecoderConfigC), _VP, _VP, _I64, _I32, _I32, _I32, _I32, _I32, C.POINTER(_VP)]),
+    "ptts_prefill_ids": (C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP, _I32, _VP]),
     "ptts_session_destroy": (C.c_int, [_VP]),
     "ptts_generate_begin": (C.c_int, [_VP, C.POINTER(GenParamsC), _VP]),
     "ptts_prefill": (C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP]),
@@ -75,6 +83,11 @@ _SIGS = {
     "ptts_dac_pack": (C.c_int, [C.POINTER(DacConfigC), _VP, _I32, _VP, _I32, _I64, _VP]),
     "ptts_dac_workspace_bytes": (C.c_int, [C.POINTER(DacConfigC), _I32, _I32, C.POINTER(_I64)]),
     "ptts_dac_decode": (C.c_int, [C.POINTER(DacConfigC), _VP, _VP, _I64, _VP, _I32, _I32, _VP, _VP]),
+    "ptts_dac_encoder_blob_bytes": (C.c_int, [C.POINTER(DacEncoderConfigC), C.POINTER(_I64)]),
+    "ptts_dac_encoder_num_tensors": (C.c_int, [C.POINTER(DacEncoderConfigC), C.POINTER(_I32)]),
+    "ptts_dac_encoder_pack": (C.c_int, [C.POINTER(DacEncoderConfigC), _VP, _I32, _VP, _I32, _I64, _VP]),
+    "ptts_dac_encoder_workspace_bytes": (C.c_int, [C.POINTER(DacEncoderConfigC), _I32, _I64, C.POINTER(_I64)]),
+    "ptts_dac_encode": (C.c_int, [C.POINTER(DacEncoderConfigC), _VP, _VP, _I64, _VP, _I32, _I64, _I32, _VP, _VP, _VP]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGS)
 

@@ -73,7 +73,8 @@ class DACConfig(_Record):
     model_type = "dac_on_the_hub"
 
     def __init__(self, num_codebooks=9, model_bitrate=8, codebook_size=1024, latent_dim=1024, frame_rate=86,
-                 sampling_rate=44100, codebook_dim=8, decoder_dim=1536, decoder_rates=(8, 8, 4, 2), **kwargs):
+                 sampling_rate=44100, codebook_dim=8, decoder_dim=1536, decoder_rates=(8, 8, 4, 2), encoder_dim=64,
+                 encoder_rates=(2, 4, 8, 8), **kwargs):
         self.codebook_size = codebook_size
         self.model_bitrate = model_bitrate
         self.latent_dim = latent_dim
@@ -85,6 +86,8 @@ class DACConfig(_Record):
         self.codebook_dim = codebook_dim
         self.decoder_dim = decoder_dim
         self.decoder_rates = list(decoder_rates)
+        self.encoder_dim = encoder_dim
+        self.encoder_rates = list(encoder_rates)
 
 
 class GenerationConfig(_Record):

@@ -1,6 +1,7 @@
 // api.cu -- the C ABI (include/ptts_b200.h): argument validation, weight packing, the generation
 // session (prefill / decode step / sample / CUDA-graph replay) and DAC decode orchestration.
 #include <cstdarg>
+#include <cstddef>
 #include <cstdlib>
 #include <cstring>
 #include <new>
@@ -53,6 +54,7 @@ struct ptts_session {
   // prefill linear layers as tcgen05 GEMMs (gemm_tc.cu) over the row-major weight copies ptts_decoder_finalize leaves in the
   // blob (layout.h rm[]); PTTS_PREFILL_TC=0 keeps the mma.sync kernel (A/B runs)
   bool prefill_tc;
+  int max_prefix;    // decoder columns ptts_prefill_ids may take (workspace rows B * (P + max_prefix))
 };
 
 extern "C" {
@@ -156,27 +158,33 @@ int ptts_decoder_finalize(const ptts_decoder_config* cfg, void* blob, void* stre
   return PTTS_OK;
 }
 
-int ptts_workspace_bytes(const ptts_decoder_config* cfg, int32_t B, int32_t P, int32_t S, int32_t max_cache_len, int64_t* out_bytes) {
+int ptts_workspace_bytes_ex(const ptts_decoder_config* cfg, int32_t B, int32_t P, int32_t S, int32_t max_cache_len, int32_t max_prefix,
+                            int64_t* out_bytes) {
   PTTS_REQUIRE(cfg && out_bytes, "null argument");
   if (int e = validate_config(*cfg)) return e;
   PTTS_REQUIRE(B > 0 && P >= 0 && S > 0 && max_cache_len > P, "workspace: need B>0, P>=0, S>0, max_cache_len>P (got %d %d %d %d)", B, P, S, max_cache_len);
-  PTTS_REQUIRE(max_cache_len <= cfg->max_positions || cfg->rope == 0 || true, "unreachable");
-  *out_bytes = make_workspace(*cfg, B, P, S, max_cache_len).total;
+  PTTS_REQUIRE(max_prefix >= 1 && P + max_prefix <= max_cache_len, "workspace: max_prefix %d out of [1, max_cache_len - P]", max_prefix);
+  *out_bytes = make_workspace(*cfg, B, P, S, max_cache_len, max_prefix).total;
   return PTTS_OK;
+}
+int ptts_workspace_bytes(const ptts_decoder_config* cfg, int32_t B, int32_t P, int32_t S, int32_t max_cache_len, int64_t* out_bytes) {
+  return ptts_workspace_bytes_ex(cfg, B, P, S, max_cache_len, 1, out_bytes);
 }
 
 // ---- session ------------------------------------------------------------------------------------
-int ptts_session_create(const ptts_decoder_config* cfg, const void* blob, void* workspace, int64_t workspace_bytes,
-                        int32_t B, int32_t P, int32_t S, int32_t max_cache_len, ptts_session** out) {
+int ptts_session_create_ex(const ptts_decoder_config* cfg, const void* blob, void* workspace, int64_t workspace_bytes,
+                           int32_t B, int32_t P, int32_t S, int32_t max_cache_len, int32_t max_prefix, ptts_session** out) {
   PTTS_REQUIRE(cfg && blob && workspace && out, "null argument");
   if (int e = validate_config(*cfg)) return e;
   PTTS_REQUIRE(B > 0 && P >= 0 && S > 0 && max_cache_len > P, "session: bad shape B=%d P=%d S=%d Tmax=%d", B, P, S, max_cache_len);
+  PTTS_REQUIRE(max_prefix >= 1 && P + max_prefix <= max_cache_len, "session: max_prefix %d out of [1, max_cache_len - P]", max_prefix);
   PTTS_REQUIRE(max_cache_len <= cfg->max_positions, "session: cache length %d exceeds max_position_embeddings %d", max_cache_len, cfg->max_positions);
   ptts_session* s = new (std::nothrow) ptts_session();
   PTTS_REQUIRE(s, "out of host memory");
   s->cfg = *cfg;
   s->L = make_layout(*cfg);
-  s->W = make_workspace(*cfg, B, P, S, max_cache_len);
+  s->W = make_workspace(*cfg, B, P, S, max_cache_len, max_prefix);
+  s->max_prefix = max_prefix;
   if (workspace_bytes < s->W.total) {
     int64_t need = s->W.total;
     delete s;
@@ -200,6 +208,10 @@ int ptts_session_create(const ptts_decoder_config* cfg, const void* blob, void* 
   s->prefill_tc = (cfg->dtype == PTTS_BF16) && env_flag("PTTS_PREFILL_TC", true);
   *out = s;
   return PTTS_OK;
+}
+int ptts_session_create(const ptts_decoder_config* cfg, const void* blob, void* workspace, int64_t workspace_bytes,
+                        int32_t B, int32_t P, int32_t S, int32_t max_cache_len, ptts_session** out) {
+  return ptts_session_create_ex(cfg, blob, workspace, workspace_bytes, B, P, S, max_cache_len, 1, out);
 }
 
 int ptts_session_destroy(ptts_session* s) {
@@ -331,13 +343,15 @@ int ptts_generate_begin(ptts_session* s, const ptts_gen_params* gen, void* strea
   return PTTS_OK;
 }
 
-// one decoder pass over q_len new positions per batch row (q_len = P+1 at prefill, 1 at decode)
-static int run_forward(ptts_session* s, cudaStream_t st, bool prefill, const void* prompt_hidden, const void* enc_hidden) {
+// one decoder pass over q_len new positions per batch row (q_len = P + n_cols at prefill, 1 at decode); col_ids: the prefill's
+// [B*K][n_cols] decoder ids, or nullptr for the single staged column
+static int run_forward(ptts_session* s, cudaStream_t st, bool prefill, const void* prompt_hidden, const void* enc_hidden,
+                       int n_cols = 1, const int64_t* col_ids = nullptr) {
   const ptts_decoder_config& c = s->cfg;
   const DecoderLayout& L = s->L;
   const WorkspaceLayout& W = s->W;
   const int B = W.B, P = W.P, S = W.S, H = L.H, D = PTTS_HEAD_DIM;
-  const int q_len = prefill ? P + 1 : 1;
+  const int q_len = prefill ? P + n_cols : 1;
   const int M = B * q_len;
   const bool pdl = !prefill;  // the one-off prefill stays on plain stream order
   const Ctrl* ctrl = prefill ? nullptr : (const Ctrl*)(s->ws + W.ctrl);
@@ -354,6 +368,7 @@ static int run_forward(ptts_session* s, cudaStream_t st, bool prefill, const voi
   ea.ctrl = ctrl;
   ea.B = B; ea.K = L.K; ea.V1 = L.V + 1; ea.H = H; ea.P = prefill ? P : 0;
   ea.pos_from_ctrl = prefill ? 0 : 1; ea.pos0 = 0; ea.prefix_len = P;
+  ea.n_cols = prefill ? n_cols : 1; ea.col_ids = prefill ? col_ids : nullptr;
   if (int e = launch_embed(ea, c.dtype, st, pdl)) return e;
   s->launches++;
 
@@ -432,22 +447,39 @@ static int run_forward(ptts_session* s, cudaStream_t st, bool prefill, const voi
              EPI_F32, nullptr, ws + W.logits, (int64_t)L.K * L.V, B, L.c_heads);
 }
 
-int ptts_prefill(ptts_session* s, const void* prompt_hidden, const int64_t* prompt_mask, const void* enc_hidden,
-                 const int64_t* enc_mask, void* stream) {
+static int prefill_common(ptts_session* s, const void* prompt_hidden, const int64_t* prompt_mask, const void* enc_hidden,
+                          const int64_t* enc_mask, const int64_t* prefix_ids, int n, cudaStream_t st) {
   PTTS_REQUIRE(s && enc_hidden, "null argument");
   if (!s->begun) return fail(PTTS_ESTATE, "ptts_prefill called before ptts_generate_begin");
   PTTS_REQUIRE(s->W.P == 0 || prompt_hidden, "prefill: prompt_hidden is required when P > 0");
-  cudaStream_t st = (cudaStream_t)stream;
+  if (prefix_ids != nullptr) {
+    // raw_ids[:, :n] = the given columns, cur_len = n: ptts_sample then appends column n
+    PTTS_CHECK_CUDA(cudaMemcpy2DAsync(s->ws + s->W.raw_ids, (size_t)s->W.raw_ld * 8, prefix_ids, (size_t)n * 8, (size_t)n * 8, s->W.BK,
+                                      cudaMemcpyDeviceToDevice, st));
+    const int cur_len = n;
+    PTTS_CHECK_CUDA(cudaMemcpyAsync(s->ws + s->W.ctrl + offsetof(Ctrl, cur_len), &cur_len, sizeof(int), cudaMemcpyHostToDevice, st));
+  }
   s->has_prompt_mask = (prompt_mask != nullptr && s->W.P > 0);
   s->has_enc_mask = (enc_mask != nullptr);
   if (s->has_prompt_mask) { if (int e = launch_mask_convert(prompt_mask, s->W.B * s->W.P, (int*)(s->ws + s->W.prompt_mask), st)) return e; }
   if (s->has_enc_mask) { if (int e = launch_mask_convert(enc_mask, s->W.B * s->W.S, (int*)(s->ws + s->W.enc_mask), st)) return e; }
-  if (int e = run_forward(s, st, true, prompt_hidden, enc_hidden)) return e;
+  if (int e = run_forward(s, st, true, prompt_hidden, enc_hidden, n, prefix_ids)) return e;
   s->prefilled = true;
   s->fused = setup_fused(s);
   // mask presence is baked into the captured graph: re-capture if it changed
   if (s->exec) { cudaGraphExecDestroy(s->exec); s->exec = nullptr; s->graph_ready = false; }
   return PTTS_OK;
+}
+int ptts_prefill(ptts_session* s, const void* prompt_hidden, const int64_t* prompt_mask, const void* enc_hidden,
+                 const int64_t* enc_mask, void* stream) {
+  return prefill_common(s, prompt_hidden, prompt_mask, enc_hidden, enc_mask, nullptr, 1, (cudaStream_t)stream);
+}
+int ptts_prefill_ids(ptts_session* s, const void* prompt_hidden, const int64_t* prompt_mask, const void* enc_hidden,
+                     const int64_t* enc_mask, const int64_t* prefix_ids, int32_t n, void* stream) {
+  PTTS_REQUIRE(s && prefix_ids, "null argument");
+  PTTS_REQUIRE(n >= 1 && n <= s->max_prefix, "prefill_ids: n = %d out of [1, max_prefix = %d]", n, s->max_prefix);
+  PTTS_REQUIRE(!s->begun || n < s->gen.max_length, "prefill_ids: n = %d leaves no new token below max_length %d", n, s->gen.max_length);
+  return prefill_common(s, prompt_hidden, prompt_mask, enc_hidden, enc_mask, prefix_ids, n, (cudaStream_t)stream);
 }
 
 int ptts_decode_forward(ptts_session* s, void* stream) {
@@ -757,6 +789,57 @@ int ptts_dac_decode(const ptts_dac_config* cfg, const void* blob, void* workspac
   }
   const int cl = C >> cfg->n_blocks;
   return conv(cur, ti + 1, ti + 2, tp(ti), nullptr, audio_out, cl, 1, Tlen, 7, 1, 1);
+}
+
+// ---- DAC encode --------------------------------------------------------------------------------
+int ptts_dac_encoder_blob_bytes(const ptts_dac_encoder_config* cfg, int64_t* out_bytes) {
+  PTTS_REQUIRE(cfg && out_bytes, "null argument");
+  if (int e = validate_dac_encoder(*cfg)) return e;
+  *out_bytes = make_dac_encoder_layout(*cfg).total;
+  return PTTS_OK;
+}
+int ptts_dac_encoder_num_tensors(const ptts_dac_encoder_config* cfg, int32_t* out) {
+  PTTS_REQUIRE(cfg && out, "null argument");
+  if (int e = validate_dac_encoder(*cfg)) return e;
+  *out = (int32_t)make_dac_encoder_layout(*cfg).t.size();
+  return PTTS_OK;
+}
+int ptts_dac_encoder_pack(const ptts_dac_encoder_config* cfg, void* blob, int32_t name_id, const void* src, int32_t src_dtype, int64_t numel,
+                          void* stream) {
+  PTTS_REQUIRE(cfg && blob && src, "null argument");
+  if (int e = validate_dac_encoder(*cfg)) return e;
+  PTTS_REQUIRE(src_dtype == PTTS_BF16 || src_dtype == PTTS_F32, "dac encoder pack: src dtype must be bf16 or f32");
+  const DacEncLayout L = make_dac_encoder_layout(*cfg);
+  PTTS_REQUIRE(name_id >= 0 && name_id < (int)L.t.size(), "dac encoder pack: tensor id %d out of range", name_id);
+  const DacTensor& t = L.t[name_id];
+  PTTS_REQUIRE(numel == t.numel, "dac encoder pack: tensor %d expects %lld elements, got %lld", name_id, (long long)t.numel, (long long)numel);
+  cudaStream_t st = (cudaStream_t)stream;
+  char* dst = (char*)blob + t.off;
+  if (t.kind == DK_PLAIN) {
+    if (int e = pack_plain(src, src_dtype, numel, dst, cfg->dtype, st)) return e;
+    const bool is_codebook = name_id >= L.first_q && (name_id - L.first_q) % 5 == 2;
+    if (!is_codebook) return PTTS_OK;
+    const int64_t k = (name_id - L.first_q) / 5, cb_bytes = (int64_t)cfg->codebook_size * cfg->codebook_dim * L.es;
+    return normalize_codebook(dst, (char*)blob + L.cb_norm + k * cb_bytes, cfg->codebook_size, cfg->codebook_dim, cfg->dtype, st);
+  }
+  if (t.off_k >= 0) {
+    if (int e = pack_conv_kmajor(src, src_dtype, (char*)blob + t.off_k, t.d0, t.d1, t.k, 0, st)) return e;
+  }
+  return pack_conv(src, src_dtype, dst, cfg->dtype, t.d0, t.d1, t.k, 0, st);
+}
+int ptts_dac_encoder_workspace_bytes(const ptts_dac_encoder_config* cfg, int32_t B, int64_t n_samples, int64_t* out_bytes) {
+  PTTS_REQUIRE(cfg && out_bytes && B > 0 && n_samples > 0, "bad argument");
+  if (int e = validate_dac_encoder(*cfg)) return e;
+  PTTS_REQUIRE(n_samples % dac_encoder_hop(*cfg) == 0, "dac encoder: n_samples %lld is not a multiple of the hop %lld", (long long)n_samples,
+               (long long)dac_encoder_hop(*cfg));
+  *out_bytes = dac_encoder_workspace(*cfg, B, n_samples);
+  return PTTS_OK;
+}
+int ptts_dac_encode(const ptts_dac_encoder_config* cfg, const void* blob, void* workspace, int64_t workspace_bytes, const void* audio, int32_t B,
+                    int64_t n_samples, int32_t n_q, int64_t* codes_out, void* z_out, void* stream) {
+  PTTS_REQUIRE(cfg && blob && workspace && audio && codes_out, "null argument");
+  if (int e = validate_dac_encoder(*cfg)) return e;
+  return dac_encode(*cfg, (const char*)blob, (char*)workspace, workspace_bytes, audio, B, n_samples, n_q, codes_out, z_out, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -13,7 +13,7 @@ import subprocess
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-SOURCES = ["api.cu", "gemm.cu", "gemm_tc.cu", "attention.cu", "embed.cu", "sample.cu", "dac.cu", "dac_tc.cu", "step.cu", "step2.cu"]
+SOURCES = ["api.cu", "gemm.cu", "gemm_tc.cu", "attention.cu", "embed.cu", "sample.cu", "dac.cu", "dac_tc.cu", "dac_enc.cu", "step.cu", "step2.cu"]
 LIB = os.path.join(HERE, "libptts_b200.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC"]

@@ -16,13 +16,6 @@
 
 namespace ptts {
 
-// snake(x) = x + (alpha + 1e-9)^-1 * sin(alpha x)^2, every op rounded to the storage dtype like torch.
-template <typename T>
-__device__ __forceinline__ float snake_fn(float x, float alpha, float inv) {
-  const float s = DT<T>::rnd(sinf(DT<T>::rnd(alpha * x)));
-  return DT<T>::rnd(x + DT<T>::rnd(inv * DT<T>::rnd(s * s)));
-}
-
 constexpr int CT_M = 64, CT_N = 64, CT_K = 16, CT_AROWS = 128, CT_MAXTAPS = 7;
 
 template <typename T>

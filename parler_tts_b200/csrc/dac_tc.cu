@@ -78,6 +78,10 @@ struct ConvTcArgs {
   const bf16* alpha_next;  // [Cout]
 };
 
+// kDown: Conv1d(k = 2s, stride s = off_step, padding s/2), the encoder's downsampling.  map_x then views the input as rows of s
+// samples ([B][Tin/s][s*Cin]); tap j of output q reads sample s*q + j - s/2 = row q + (j + s/2)/s - 1 at column ((j + s/2) % s)*Cin,
+// so every (tap, 64-channel chunk) is still one TMA box and the box's zero fill outside [0, Tin/s) is the convolution's padding.
+template <bool kDown>
 __global__ void __launch_bounds__(TC_THREADS, 2)
 conv_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_w, const ConvTcArgs p) {
   extern __shared__ __align__(1024) unsigned char smem[];
@@ -121,7 +125,12 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant_
         unsigned char* a_dst = stages + (size_t)s * stage_bytes;
         unsigned char* b_dst = a_dst + a_bytes;
         tc_mbar_expect(&full[s], (uint32_t)(a_bytes + b_bytes));
-        tma_load_3d(a_dst, &map_x, kc * TC_K, q0 + p.off_base + j * p.off_step, b, &full[s]);
+        if constexpr (kDown) {
+          const int sh = j + (p.off_step >> 1);
+          tma_load_3d(a_dst, &map_x, (sh % p.off_step) * p.Cin + kc * TC_K, q0 + sh / p.off_step - 1, b, &full[s]);
+        } else {
+          tma_load_3d(a_dst, &map_x, kc * TC_K, q0 + p.off_base + j * p.off_step, b, &full[s]);
+        }
         tma_load_3d(b_dst, &map_w, kc * TC_K, n0, p.wt_base + phase * p.wt_phase_step + j * p.wt_step, &full[s]);
       }
     }
@@ -262,6 +271,20 @@ static int encode_map(CUtensorMap* m, const void* base, uint64_t d0, uint64_t d1
   return PTTS_OK;
 }
 
+template <bool kDown>
+static int launch_tc(const CUtensorMap& mx, const CUtensorMap& mw, const ConvTcArgs& p, dim3 grid, cudaStream_t st) {
+  const int stage_bytes = (TC_M * TC_K * 2 + p.n_tile * TC_K * 2 + 1023) & ~1023;
+  const size_t smem = (size_t)TC_STAGES * stage_bytes + 128 + 3 * 256 * 2;
+  static bool attr = false;
+  if (!attr) {
+    PTTS_CHECK_CUDA(cudaFuncSetAttribute(conv_tc_kernel<kDown>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024));
+    attr = true;
+  }
+  conv_tc_kernel<kDown><<<grid, TC_THREADS, smem, st>>>(mx, mw, p);
+  PTTS_LAUNCH_CHECK();
+  return PTTS_OK;
+}
+
 bool conv_tc_supported(int Cin, int Cout) {
   return Cin % 8 == 0 && Cin >= 64 && Cout % 32 == 0 && Cout >= 32;  // row pitch multiple of 16 B; epilogue works in 32-column chunks
 }
@@ -286,17 +309,28 @@ int launch_conv_tc(const ConvArgs& a, const void* w_kmajor, int taps_total, cons
   CUtensorMap mx, mw;
   if (int e = make_map(&mx, a.x, (uint64_t)a.Cin, (uint64_t)a.Tin, (uint64_t)B, TC_M)) return e;
   if (int e = make_map(&mw, w_kmajor, (uint64_t)a.Cin, (uint64_t)a.Cout, (uint64_t)taps_total, (uint32_t)p.n_tile)) return e;
-  const int stage_bytes = (TC_M * TC_K * 2 + p.n_tile * TC_K * 2 + 1023) & ~1023;
-  const size_t smem = (size_t)TC_STAGES * stage_bytes + 128 + 3 * 256 * 2;
-  static bool attr = false;
-  if (!attr) {
-    PTTS_CHECK_CUDA(cudaFuncSetAttribute(conv_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024));
-    attr = true;
-  }
   dim3 grid((a.q_count + TC_M - 1) / TC_M, a.Cout / p.n_tile, B * a.n_phase);
-  conv_tc_kernel<<<grid, TC_THREADS, smem, st>>>(mx, mw, p);
-  PTTS_LAUNCH_CHECK();
-  return PTTS_OK;
+  return launch_tc<false>(mx, mw, p, grid, st);
+}
+
+bool conv_tc_down_supported(int Cin, int Cout) { return Cin % TC_K == 0 && conv_tc_supported(Cin, Cout); }
+
+// x: [B][Tin][Cin] bf16 (Tin % s == 0), w: [2s][Cout][Cin] bf16 -> [B][Tin/s][Cout]
+int launch_conv_tc_down(const void* x, const void* w_kmajor, const void* bias, const void* alpha_next, void* out_raw, void* out_act,
+                        int Cin, int Cout, int Tin, int s, int B, cudaStream_t st) {
+  PTTS_REQUIRE(conv_tc_down_supported(Cin, Cout) && s >= 2 && s % 2 == 0 && Tin % s == 0, "conv_tc_down: Cin=%d Cout=%d s=%d Tin=%d unsupported", Cin, Cout, s, Tin);
+  ConvTcArgs p{};
+  p.Cin = Cin; p.Cout = Cout; p.Tin = Tin; p.Tout = Tin / s; p.q_count = Tin / s;
+  p.n_taps = 2 * s; p.off_base = 0; p.off_step = s; p.wt_base = 0; p.wt_step = 1;
+  p.n_phase = 1; p.wt_phase_step = 0; p.o_mul = 1; p.o_add = 0; p.o_phase_step = 0;
+  p.n_tile = conv_tc_ntile(Cout);
+  p.tmem_cols = p.n_tile <= 32 ? 32 : (p.n_tile <= 64 ? 64 : (p.n_tile <= 128 ? 128 : 256));
+  p.bias = (const bf16*)bias; p.res = nullptr; p.out_raw = (bf16*)out_raw; p.out_act = (bf16*)out_act; p.alpha_next = (const bf16*)alpha_next;
+  CUtensorMap mx, mw;
+  if (int e = make_map(&mx, x, (uint64_t)s * Cin, (uint64_t)(Tin / s), (uint64_t)B, TC_M)) return e;
+  if (int e = make_map(&mw, w_kmajor, (uint64_t)Cin, (uint64_t)Cout, (uint64_t)(2 * s), (uint32_t)p.n_tile)) return e;
+  dim3 grid((p.q_count + TC_M - 1) / TC_M, Cout / p.n_tile, B);
+  return launch_tc<true>(mx, mw, p, grid, st);
 }
 
 // weight repack for the tensor-core path: Conv1d [co][ci][k] / ConvTranspose1d [ci][co][k] -> [k][co][ci] bf16

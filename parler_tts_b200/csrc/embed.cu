@@ -14,7 +14,7 @@ __global__ void __launch_bounds__(128) embed_kernel(EmbedArgs p) {
   pdl_launch_dependents();
   pdl_wait();
   if (p.ctrl != nullptr && p.ctrl->active == 0) return;
-  const int rows_per_b = p.P + 1;
+  const int rows_per_b = p.P + p.n_cols;
   const int b = blockIdx.x / rows_per_b, j = blockIdx.x - b * rows_per_b;
   const int position = p.pos_from_ctrl ? (p.prefix_len + p.ctrl->cur_len - 1) : (p.pos0 + j);
   const T* tables = reinterpret_cast<const T*>(p.tables);
@@ -27,7 +27,7 @@ __global__ void __launch_bounds__(128) embed_kernel(EmbedArgs p) {
     } else {
       v = 0.f;
       for (int k = 0; k < p.K; k++) {
-        const int id = p.ids[b * p.K + k];
+        const int id = p.col_ids != nullptr ? (int)p.col_ids[(size_t)(b * p.K + k) * p.n_cols + (j - p.P)] : p.ids[b * p.K + k];
         const float e = DT<T>::to_f(tables[((size_t)k * p.V1 + id) * p.H + c]);
         v = (k == 0) ? e : DT<T>::rnd(v + e);  // sum([...]) accumulates left to right in the model dtype
       }
@@ -39,7 +39,7 @@ __global__ void __launch_bounds__(128) embed_kernel(EmbedArgs p) {
 
 int launch_embed(const EmbedArgs& a, int dtype, cudaStream_t st, bool pdl) {
   cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(a.B * (a.P + 1));
+  cfg.gridDim = dim3(a.B * (a.P + a.n_cols));
   cfg.blockDim = dim3(128);
   cfg.stream = st;
   cudaLaunchAttribute at[1];

@@ -57,6 +57,8 @@ struct EmbedArgs {
   const Ctrl* ctrl;
   int B, K, V1, H, P;  // P = prefix rows per batch in THIS call (0 at decode)
   int pos_from_ctrl, pos0, prefix_len;  // decode: position = prefix_len + cur_len - 1
+  int n_cols;              // decoder columns per batch row in THIS call (1 at decode; n for a voice-prompt prefill)
+  const int64_t* col_ids;  // [B*K][n_cols] ids of those columns, or nullptr: one column from `ids`
 };
 int launch_embed(const EmbedArgs& a, int dtype, cudaStream_t st, bool pdl);
 

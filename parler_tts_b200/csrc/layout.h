@@ -140,7 +140,7 @@ static inline bool matrix_slot(const DecoderLayout& l, int tensor_id, int index,
 
 // ---- workspace ----------------------------------------------------------------------------------
 struct WorkspaceLayout {
-  int B, P, S, Tmax, Mmax, BK;
+  int B, P, S, Tmax, Mmax, BK;    // Mmax = B * (P + max_prefix) rows of the first forward
   int64_t ctrl, progress, gen, raw_ids, cur_ids, eos_seen, unfinished, first_unf, prompt_mask, enc_mask;
   int64_t x, qkv, attn, qc, hbuf, hidden, logits, scores, cross_tmp, cross_kv, self_kv;
   int64_t img_x, img_attn, img_h;  // fused step kernel: activations as tile images [chunk][32][H + 8] (step.cu stage_tile)
@@ -151,11 +151,12 @@ struct WorkspaceLayout {
   int64_t total;
 };
 
-static inline WorkspaceLayout make_workspace(const ptts_decoder_config& c, int B, int P, int S, int Tmax) {
+// max_prefix: decoder columns the first forward may take (1 = the BOS column; more for a voice-prompt prefix, ptts_prefill_ids)
+static inline WorkspaceLayout make_workspace(const ptts_decoder_config& c, int B, int P, int S, int Tmax, int max_prefix = 1) {
   DecoderLayout l = make_layout(c);
   WorkspaceLayout w{};
   w.B = B; w.P = P; w.S = S; w.Tmax = Tmax; w.BK = B * c.num_codebooks;
-  w.Mmax = B * (P + 1);
+  w.Mmax = B * (P + max_prefix);
   int64_t o = 0;
   auto take = [&](int64_t bytes) { int64_t r = o; o = align_up(o + bytes, 256); return r; };
   w.ctrl = take(sizeof(Ctrl));

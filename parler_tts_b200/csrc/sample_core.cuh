@@ -343,7 +343,7 @@ __device__ __forceinline__ void sample_rows_cta(const SampleArgs& p, const ptts_
   if (tid < R && my_valid) {
     const int b = my_row / p.K, k = my_row - b * p.K;
     int t = my_tok;
-    if (forced != nullptr) t = (int)forced[my_row];
+    if (forced != nullptr && forced[my_row] >= 0) t = (int)forced[my_row];   // negative: draw this row (ptts_sample)
     if (!t_unf) t = p.pad;  // next_tokens * unfinished + pad * (1 - unfinished)
     p.raw_ids[(size_t)my_row * p.raw_ld + cur_len] = t;
     if (t == p.eos && t_es == 0) p.eos_seen[my_row] = cur_len + 1;

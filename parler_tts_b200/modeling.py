@@ -184,13 +184,13 @@ class DecoderEngine:
             return sd[f"{prefix}lm_heads.weight"][k * V:(k + 1) * V]
         raise ValueError(f"missing weight {prefix}lm_heads.{k}.weight")
 
-    def session(self, B: int, P: int, S: int, max_cache_len: int) -> "GenSession":
+    def session(self, B: int, P: int, S: int, max_cache_len: int, max_prefix: int = 1) -> "GenSession":
         key = (B, P, S)
         s = self._sessions.get(key)
-        if s is None or s.max_cache_len < max_cache_len:
+        if s is None or s.max_cache_len < max_cache_len or s.max_prefix < max_prefix:
             if s is not None:
                 s.close()
-            s = GenSession(self, B, P, S, max_cache_len)
+            s = GenSession(self, B, P, S, max_cache_len, max_prefix)
             self._sessions = {key: s}  # keep one live session (the reference keeps one `_cache`, :3254-3309)
         return s
 
@@ -198,15 +198,15 @@ class DecoderEngine:
 class GenSession:
     """Device-resident generation state for (B, P, S): KV caches, token history, processor state."""
 
-    def __init__(self, eng: DecoderEngine, B: int, P: int, S: int, max_cache_len: int):
-        self.eng, self.B, self.P, self.S, self.max_cache_len = eng, B, P, S, max_cache_len
+    def __init__(self, eng: DecoderEngine, B: int, P: int, S: int, max_cache_len: int, max_prefix: int = 1):
+        self.eng, self.B, self.P, self.S, self.max_cache_len, self.max_prefix = eng, B, P, S, max_cache_len, max_prefix
         lib = _lib.lib()
         n = C.c_int64()
-        _lib.check(lib.ptts_workspace_bytes(C.byref(eng.c), B, P, S, max_cache_len, C.byref(n)))
+        _lib.check(lib.ptts_workspace_bytes_ex(C.byref(eng.c), B, P, S, max_cache_len, max_prefix, C.byref(n)))
         self.ws = torch.zeros(n.value, dtype=torch.uint8, device=eng.device)
         h = C.c_void_p()
-        _lib.check(lib.ptts_session_create(C.byref(eng.c), _lib.ptr(eng.blob), _lib.ptr(self.ws), n.value, B, P, S,
-                                           max_cache_len, C.byref(h)))
+        _lib.check(lib.ptts_session_create_ex(C.byref(eng.c), _lib.ptr(eng.blob), _lib.ptr(self.ws), n.value, B, P, S,
+                                              max_cache_len, max_prefix, C.byref(h)))
         self.h = h
         self.K, self.V = eng.cfg.num_codebooks, eng.cfg.vocab_size
         self._keep: list[Any] = []
@@ -274,7 +274,8 @@ class GenSession:
         _lib.check(_lib.lib().ptts_generate_begin(self.h, C.byref(g), _lib.stream_ptr()))
         self.max_length = int(max_length)
 
-    def prefill(self, prompt_hidden, prompt_mask, enc_hidden, enc_mask):
+    def prefill(self, prompt_hidden, prompt_mask, enc_hidden, enc_mask, prefix_ids=None):
+        """prefix_ids: None (the BOS column begin() staged) or [B*K, n] delay-patterned decoder ids (ptts_prefill_ids)."""
         dt, dev = self.eng.dtype, self.eng.device
         H = self.eng.cfg.hidden_size
         enc_hidden = enc_hidden.to(device=dev, dtype=dt).contiguous()
@@ -288,9 +289,19 @@ class GenSession:
                 raise ValueError(f"prompt states must be [{self.B}, {self.P}, {H}], got {tuple(prompt_hidden.shape)}")
         pm = None if prompt_mask is None else prompt_mask.to(device=dev, dtype=torch.int64).contiguous()
         em = None if enc_mask is None else enc_mask.to(device=dev, dtype=torch.int64).contiguous()
-        self._keep = [prompt_hidden, enc_hidden, pm, em]
-        _lib.check(_lib.lib().ptts_prefill(self.h, _lib.ptr(prompt_hidden) if self.P > 0 else None, _lib.ptr(pm),
-                                           _lib.ptr(enc_hidden), _lib.ptr(em), _lib.stream_ptr()))
+        if prefix_ids is None:
+            self._keep = [prompt_hidden, enc_hidden, pm, em]
+            _lib.check(_lib.lib().ptts_prefill(self.h, _lib.ptr(prompt_hidden) if self.P > 0 else None, _lib.ptr(pm),
+                                               _lib.ptr(enc_hidden), _lib.ptr(em), _lib.stream_ptr()))
+            return
+        ids = prefix_ids.to(device=dev, dtype=torch.int64).contiguous()
+        if ids.dim() != 2 or ids.shape[0] != self.B * self.K:
+            raise ValueError(f"prefix ids must be [{self.B * self.K}, n], got {tuple(ids.shape)}")
+        if bool(((ids < 0) | (ids > self.V)).any()):
+            raise ValueError(f"prefix ids must lie in [0, {self.V}] (the embedding tables have vocab_size + 1 rows)")
+        self._keep = [prompt_hidden, enc_hidden, pm, em, ids]
+        _lib.check(_lib.lib().ptts_prefill_ids(self.h, _lib.ptr(prompt_hidden) if self.P > 0 else None, _lib.ptr(pm),
+                                               _lib.ptr(enc_hidden), _lib.ptr(em), _lib.ptr(ids), ids.shape[1], _lib.stream_ptr()))
 
     def decode_forward(self):
         _lib.check(_lib.lib().ptts_decode_forward(self.h, _lib.stream_ptr()))
@@ -326,9 +337,10 @@ class ParlerTTSCache:
     def __init__(self, session: "GenSession"):
         self.session = session
         self.steps = 0
+        self.n_first = 1   # decoder columns of the first call (> 1: a voice-prompt prefix)
 
     def get_seq_length(self) -> int:
-        return self.session.P + 1 + self.steps
+        return self.session.P + self.n_first + self.steps
 
     def get_max_cache_shape(self) -> int:
         return self.session.max_cache_len
@@ -364,12 +376,16 @@ class ParlerTTSForCausalLM:
           Only the LAST position's logits are materialised (what `_sample` reads): shape [B*K, 1, V], not [B*K, P+1, V].
         * later calls: the ids are appended (ptts_sample with forced tokens) and one cached step runs on the fused kernel
           (ptts_decode_forward).
-        Inputs longer than one column, `inputs_embeds`, `labels` and `use_cache=False` belong to training / the no-cache path and
-        are outside this operator (ValueError)."""
+        * the first call may also take input_ids [B*K, n] (a delay-patterned voice-prompt prefix, column 0 = BOS): the n columns go
+          through ptts_prefill_ids in one forward and get_seq_length() counts them.
+        Later calls with more than one column, `inputs_embeds`, `labels` and `use_cache=False` belong to training / the no-cache
+        path and are outside this operator (ValueError)."""
         if kwargs.get("inputs_embeds") is not None or kwargs.get("labels") is not None or not use_cache:
             raise ValueError("ParlerTTSForCausalLM.forward on the B200 path is the cached decode-step operator: input_ids [B*K, 1], use_cache=True")
-        if input_ids is None or input_ids.dim() != 2 or input_ids.shape[1] != 1 or input_ids.shape[0] % self.num_codebooks != 0:
-            raise ValueError(f"input_ids must be [batch * num_codebooks, 1], got {None if input_ids is None else tuple(input_ids.shape)}")
+        n_cols = 1 if past_key_values is not None else (input_ids.shape[-1] if input_ids is not None and input_ids.dim() == 2 else 0)
+        if input_ids is None or input_ids.dim() != 2 or input_ids.shape[1] != n_cols or n_cols < 1 or input_ids.shape[0] % self.num_codebooks != 0:
+            raise ValueError(f"input_ids must be [batch * num_codebooks, 1] (or [batch * num_codebooks, n] on the first call), got "
+                             f"{None if input_ids is None else tuple(input_ids.shape)}")
         B = input_ids.shape[0] // self.num_codebooks
         ids = input_ids[:, 0].to(self.device, torch.int64).contiguous()
         if past_key_values is None:
@@ -378,12 +394,14 @@ class ParlerTTSForCausalLM:
             S = encoder_hidden_states.shape[1]
             P = 0 if prompt_hidden_states is None else prompt_hidden_states.shape[1]
             cap = int(max_cache_len or self.config.max_position_embeddings)
-            sess = GenSession(self.engine, B, P, S, cap)   # an independent cache, not the engine's shared generate() session
+            sess = GenSession(self.engine, B, P, S, cap, max_prefix=n_cols)   # an independent cache, not generate()'s shared session
             sess.begin(cap - P, do_sample=False)
             if not bool((ids == self.config.bos_token_id).all()):
                 raise ValueError("the first call must feed the decoder start (BOS) column")
-            sess.prefill(prompt_hidden_states, prompt_attention_mask if P > 0 else None, encoder_hidden_states, encoder_attention_mask)
+            sess.prefill(prompt_hidden_states, prompt_attention_mask if P > 0 else None, encoder_hidden_states, encoder_attention_mask,
+                         prefix_ids=input_ids if n_cols > 1 else None)
             past_key_values = ParlerTTSCache(sess)
+            past_key_values.n_first = n_cols
         else:
             if not isinstance(past_key_values, ParlerTTSCache) or past_key_values.session.B != B:
                 raise ValueError("past_key_values must be the ParlerTTSCache returned by the first call (same batch)")
@@ -624,20 +642,29 @@ class ParlerTTSForConditionalGeneration:
         return 32
 
     def _run_token_loop(self, enc_hidden, attention_mask, prompt_hidden, prompt_mask, *, gc, max_length, seed, suppress_special, row_base,
-                        streamer=None, custom=None):
-        """begin + prefill + the token loop of one session; returns the raw token matrix [B * K, generated length]."""
+                        streamer=None, custom=None, prefix=None, forced=None):
+        """begin + prefill + the token loop of one session; returns the raw token matrix [B * K, generated length].
+
+        prefix [B*K, n]: the model's first n input columns of a voice-prompt continuation (delay-patterned, column 0 = BOS);
+        forced [B*K, max_length]: the prompt codes the delay pattern puts after the prefix (codebook k: columns n .. n+k-1), -1
+        elsewhere."""
         d = self.config.decoder
         K = d.num_codebooks
         B, S, _ = enc_hidden.shape
         P = 0 if prompt_hidden is None else prompt_hidden.shape[1]
-        sess = self.decoder.engine.session(B, P, S, P + max_length)
+        n = 1 if prefix is None else prefix.shape[1]
+        sess = self.decoder.engine.session(B, P, S, P + max_length, max_prefix=n)
+        # MinNewTokensLengthLogitsProcessor skips the n prompt columns (:3540-3547); the kernel tests cur_len - 1 < min_new_tokens
+        min_new = gc.min_new_tokens or 0
+        if min_new > 0:
+            min_new += n - 1
         sess.begin(max_length, do_sample=gc.do_sample, temperature=gc.temperature, top_k=gc.top_k if gc.do_sample else 0,
-                   top_p=gc.top_p, min_new_tokens=gc.min_new_tokens or 0, seed=seed, suppress_special=suppress_special,
+                   top_p=gc.top_p, min_new_tokens=min_new, seed=seed, suppress_special=suppress_special,
                    codebook_size=self.config.audio_encoder.codebook_size, row_base=row_base)
         if streamer is not None:
             delayed = torch.full((B * K, 1), d.bos_token_id, dtype=torch.int64)
             streamer.put(delayed)
-        sess.prefill(prompt_hidden, prompt_mask, enc_hidden, attention_mask)
+        sess.prefill(prompt_hidden, prompt_mask, enc_hidden, attention_mask, prefix_ids=prefix)
         if custom is not None:
             self._host_driven_loop(sess, gc, max_length, custom[0], custom[1], streamer, seed)
         elif streamer is not None:
@@ -653,8 +680,17 @@ class ParlerTTSForConditionalGeneration:
                 streamer.put(sess.raw_ids[:, col].cpu())
             streamer.end()
         else:
-            sess.sample()
-            steps_left = max_length - 2
+            # After a prefix, the first K-1 columns run one step at a time with the pattern's prompt codes forced (a negative entry
+            # draws).  That matches the reference in output and in stopping: the Parler processor lets codebook k draw EOS at
+            # column n + k at the earliest and first_codebooks_unfinished moves by at most one per step, so a forced cell never
+            # holds a drawn EOS there; the reference's history differs only in cells its final mask overwrites.
+            sess.sample(None if prefix is None else forced[:, n])
+            col = n + 1
+            while prefix is not None and col < min(n + K - 1, max_length):
+                sess.decode_forward()
+                sess.sample(forced[:, col])
+                col += 1
+            steps_left = max_length - col
             # no per-step host sync: enqueue graph replays in chunks and poll the device `active` flag between chunks
             chunk = 64
             while steps_left > 0:
@@ -697,8 +733,14 @@ class ParlerTTSForConditionalGeneration:
             raise ValueError("Got incompatible mode for generation, should be one of greedy or sampling. "
                              "Ensure that beam search is de-activated by setting `num_beams=1` and `num_beam_groups=1`.")
         custom_loop = bool(logits_processor) or bool(stopping_criteria)   # merged with the built-in ones like :3540-3552
-        if mk.get("decoder_input_ids") is not None or mk.get("input_values") is not None:
-            raise ValueError("audio-prompt continuation (decoder_input_ids / input_values) is outside this path")
+        prefix = mk.get("decoder_input_ids")
+        if (prefix is not None or mk.get("input_values") is not None) and (streamer is not None or custom_loop):
+            raise ValueError("an audio prompt (decoder_input_ids / input_values) together with streamer= or user logits_processor / "
+                             "stopping_criteria is not supported")
+        if prefix is None and mk.get("input_values") is not None:
+            # :3442-3446: the codec's codes of the reference audio, [B, K, T_a] -> [B*K, T_a]
+            codes = self.audio_encoder.encode(mk["input_values"], n_quantizers=self.config.decoder.num_codebooks).audio_codes[0]
+            prefix = codes.reshape(-1, codes.shape[-1])
         input_ids = mk.get("input_ids", inputs)
         attention_mask = mk.get("attention_mask")
         enc = mk.get("encoder_outputs")
@@ -718,16 +760,30 @@ class ParlerTTSForConditionalGeneration:
         prompt_mask = mk.get("prompt_attention_mask") if prompt_hidden is not None else None
         P = 0 if prompt_hidden is None else prompt_hidden.shape[1]
 
-        # generated length (:3458-3469): max_new_tokens wins over max_length; input_ids_length == 1
-        if gc.max_new_tokens is not None:
-            max_length = int(gc.max_new_tokens) + 1
-        else:
-            max_length = int(user_max_length if user_max_length is not None else gc.max_length)
-        if max_length < 2:
-            raise ValueError(f"max_length must allow at least one new token, got {max_length}")
         d = self.config.decoder
         K = d.num_codebooks
+        if prefix is not None:
+            prefix = prefix.to(self.device, torch.int64)
+            if prefix.dim() != 2 or prefix.shape[0] != B * K or prefix.shape[1] < 1:
+                raise ValueError(f"decoder_input_ids must be [{B * K}, n], got {tuple(prefix.shape)}")
+            if bool((prefix[:, 0] != d.bos_token_id).all()):   # :3017-3031: BOS column unless every row already starts with it
+                prefix = torch.cat([torch.full((B * K, 1), d.bos_token_id, dtype=torch.int64, device=self.device), prefix], dim=1)
+        n = 1 if prefix is None else prefix.shape[1]
+        # generated length (:3458-3469): max_new_tokens wins over max_length; input_ids_length == n
+        if gc.max_new_tokens is not None:
+            max_length = int(gc.max_new_tokens) + n
+        else:
+            max_length = int(user_max_length if user_max_length is not None else gc.max_length)
+        if max_length < n + 1:
+            raise ValueError(f"max_length must allow at least one new token, got {max_length} for {n} decoder input columns")
         run = dict(gc=gc, max_length=max_length, seed=seed, suppress_special=suppress_special)
+        pattern = forced = None
+        if prefix is not None:
+            # :3523-3528: the model's first input is the first n columns of the pattern built from the whole prefix; the prompt codes
+            # it shifts past column n are forced where the BOS-only pattern the device applies has a free cell
+            prefix, pattern = build_delay_pattern_mask(prefix, d.bos_token_id, d.pad_token_id, max_length, K)
+            _, device_pattern = build_delay_pattern_mask(prefix[:, :1], d.bos_token_id, d.pad_token_id, max_length, K)
+            forced = torch.where((device_pattern == -1) & (pattern != -1), pattern, torch.full_like(pattern, -1))
         limit = self._fused_batch_limit()
         if limit is not None and B > limit and not custom_loop and streamer is None:
             # The fused decode-step kernels hold one 32-row tile: a larger batch runs as consecutive shards of <= 32 utterances through
@@ -736,17 +792,25 @@ class ParlerTTSForConditionalGeneration:
             parts = []
             for b0 in range(0, B, limit):
                 sl = slice(b0, min(B, b0 + limit))
+                rows = slice(sl.start * K, sl.stop * K)
                 parts.append(self._run_token_loop(enc_hidden[sl], None if attention_mask is None else attention_mask[sl],
                                                   None if prompt_hidden is None else prompt_hidden[sl],
-                                                  None if prompt_mask is None else prompt_mask[sl], row_base=row_base + b0 * K, **run))
+                                                  None if prompt_mask is None else prompt_mask[sl], row_base=row_base + b0 * K,
+                                                  prefix=None if prefix is None else prefix[rows].contiguous(),
+                                                  forced=None if forced is None else forced[rows].contiguous(), **run))
             n = max(t.shape[1] for t in parts)
             output_ids = torch.cat([torch.nn.functional.pad(t, (0, n - t.shape[1]), value=d.pad_token_id) for t in parts], dim=0)
         else:
             output_ids = self._run_token_loop(enc_hidden, attention_mask, prompt_hidden, prompt_mask, row_base=row_base, streamer=streamer,
-                                              custom=(logits_processor or [], stopping_criteria or []) if custom_loop else None, **run)
+                                              custom=(logits_processor or [], stopping_criteria or []) if custom_loop else None,
+                                              prefix=prefix, forced=forced, **run)
 
-        # apply the stashed delay mask, then keep only the free cells (:3586-3597)
-        _, full_mask = build_delay_pattern_mask(output_ids[:, :1], d.bos_token_id, d.pad_token_id, max_length, K)
+        # apply the stashed delay mask (built from the whole prefix: the output starts with the prompt's own frames), then keep only
+        # the free cells (:3586-3597)
+        if pattern is not None:
+            full_mask = pattern
+        else:
+            _, full_mask = build_delay_pattern_mask(output_ids[:, :1], d.bos_token_id, d.pad_token_id, max_length, K)
         output_ids = apply_delay_pattern_mask(output_ids, full_mask)
         _, mask = build_delay_pattern_mask(output_ids[:, :1], d.bos_token_id, d.pad_token_id, output_ids.shape[1], K)
         keep = (mask != d.bos_token_id) & (mask != d.pad_token_id)
